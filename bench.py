@@ -27,8 +27,18 @@ one pass of the filter over the whole recording.
   channel-sharded) and a cfg5 candidate sweep (1e5 periods, winner by one (error, index)
   pair per rank).
 
+``--steps K`` is the number of timed passes of ``value``, ``e2e`` (per window), each
+``e2e_variants`` window and ``find_period`` (its fp32 mode too); the strong-scaling,
+``standardise`` and power-capped (``roofline.sustained``) figures time fixed counts of their own.
+
 ``--impl reference`` times the unmodified reference's ``PARRM.filter_data()`` on this host's
 cores on bounded samples of the same workload; rank 0 only; it maps no library of this repo.
+
+``--dump-outputs DIR`` (rank 0) writes, after the timed steps, what the last of them computed:
+``filter_data.npy``, rows ``DUMP_ROWS`` of the headline's filtered recording (float64
+[4, 1 200 000]), and ``find_period_errors.npy``, the evaluator's fit errors of its last timed
+step (float64).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 
 Multi-GPU (torchrun, one rank per GPU) goes through the product's own sharding API:
 ``pyparrm_b200.enable_sharding()`` + ``PARRM.filter_data()`` / ``PARRM.find_period()``.  Weak
@@ -57,6 +67,10 @@ HALF_WIDTH = 2000
 WORKLOAD = ("cfg2: synthetic 64-ch LFP, 2 kHz, 130 Hz DBS artefact, 10 min (64 x 1.2M f64), "
             "filter_half_width=2000, bidirectional")
 BYTES_PER_CHANNEL_SAMPLE = 16.0  # float64: 8 read + 8 written (SURVEY 8(d))
+# --dump-outputs keeps these whole rows of the 614 MB filtered recording (38.4 MB): every
+# sample of a row, the edges included, where the taps run off the recording
+DUMP_ROWS = np.sort(np.random.default_rng(0).choice(N_CHANS, 4, replace=False))
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 # ----------------------------------------------------------------------------- helpers
@@ -177,6 +191,19 @@ def barrier(dist):
     if dist is not None:
         dist.barrier()
     torch.cuda.synchronize()
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Write each array as ``directory/<name>.npy``, so that two builds can be compared output
+    for output on the same seeded inputs."""
+    nbytes = sum(a.nbytes for a in arrays.values())
+    if nbytes > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {nbytes} bytes, more than {DUMP_LIMIT_BYTES}")
+    for name, array in arrays.items():
+        if array.dtype not in (np.float32, np.float64):
+            raise TypeError(f"--dump-outputs: {name} is {array.dtype}, not float32 or float64")
+    for name, array in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), array)
 
 
 # ----------------------------------------------------------------------------- CPU legs
@@ -454,6 +481,9 @@ def run_b200(args):
         dev_seconds = max_over_ranks(dist, start.elapsed_time(stop) * 1e-3)
         kernel_seconds = start.elapsed_time(stop) * 1e-3 / args.steps  # one launch per step
         rank_ms = [round(1e3 * v, 4) for v in all_ranks(dist, kernel_seconds)]
+        dumped = {}
+        if args.dump_outputs and rank == 0:
+            dumped["filter_data"] = d_y[DUMP_ROWS.tolist()].cpu().numpy()
 
         # the same pass after half a second of back-to-back passes: the GPU at its power cap
         t_hot = time.perf_counter()
@@ -474,8 +504,7 @@ def run_b200(args):
         # ---- e2e: public API, host in / host out (sharded through enable_sharding) ---
         for _ in range(min(args.warmup, 3)):
             parrm.filter_data()
-        e2e_steps = max(3, min(args.steps, 20))
-        # back-to-back windows of e2e_steps passes, all reported; the line's e2e is the fastest
+        # back-to-back windows of --steps passes, all reported; the line's e2e is the fastest
         # one.  The path is bound by the host's PCIe / memory system, which this process shares
         # with whatever else runs on the box, so windows repeat -- at most five -- until the two
         # fastest agree within 3 %.  (A result kept alive across windows makes the next window
@@ -485,7 +514,7 @@ def run_b200(args):
         out = None
         for _ in range(5):
             out = None
-            seconds, out = timed_api_passes(dist, parrm.filter_data, e2e_steps)
+            seconds, out = timed_api_passes(dist, parrm.filter_data, args.steps)
             e2e_windows.append(seconds)
             e2e_passes.append(timed_api_passes.last_pass_ms)
             best = sorted(e2e_windows)
@@ -495,7 +524,7 @@ def run_b200(args):
         assert tuple(parrm.filter_shard) == (c0, c1, 0, N_SAMPLES)
 
         # ---- find_period evaluator (second metric) + the sharded search API ----------
-        search = bench_search(engine, dist, world, rank, args)
+        search = bench_search(engine, dist, world, rank, args, dumped)
 
         # ---- strong-scaling cases (device resident) --------------------------------
         strong = bench_strong(engine, dist, world, rank)
@@ -509,7 +538,7 @@ def run_b200(args):
 
     variants, cfg1 = {}, None
     if world == 1:
-        variants = bench_e2e_variants(engine, data, taps, e2e_steps, period)
+        variants = bench_e2e_variants(engine, data, taps, args.steps, period)
         cfg1 = bench_cfg1(engine)
     if pin is not None:
         pin.release()
@@ -517,6 +546,8 @@ def run_b200(args):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
 
     cpu = cpu_filter_baseline(data, period) if world == 1 else None
     achieved = BYTES_PER_CHANNEL_SAMPLE * units / kernel_seconds / 1e9
@@ -545,10 +576,10 @@ def run_b200(args):
         },
         "clocks": clocks.summary(),
         "e2e": {
-            "value": world * units * e2e_steps / e2e_seconds, "unit": "channel-samples/s",
+            "value": world * units * args.steps / e2e_seconds, "unit": "channel-samples/s",
             "h2d_bytes_per_step": units * 8, "d2h_bytes_per_step": units * 8,
-            "steps": e2e_steps, "ms_per_step": 1e3 * e2e_seconds / e2e_steps,
-            "windows_ms_per_step": [round(1e3 * w / e2e_steps, 3) for w in e2e_windows],
+            "steps": args.steps, "ms_per_step": 1e3 * e2e_seconds / args.steps,
+            "windows_ms_per_step": [round(1e3 * w / args.steps, 3) for w in e2e_windows],
             "slowest_window_pass_ms": e2e_passes[int(np.argmax(e2e_windows))],
             "pcie_floor": recorded_pcie_floor(world),
             "api": ("PARRM.filter_data() under enable_sharding(gather='none'); this rank's rows "
@@ -876,9 +907,10 @@ def bench_strong(engine, dist, world, rank):
     return out
 
 
-def bench_search(engine, dist, world, rank, args):
+def bench_search(engine, dist, world, rank, args, dumped):
     """Evaluator throughput on the run-3 shape of the cfg2 recording (candidates sharded over
-    ranks by the product's evaluate_sharded), then the whole search through the public API."""
+    ranks by the product's evaluate_sharded), then the whole search through the public API.
+    With --dump-outputs the errors of the last timed step go into ``dumped``."""
     import torch
 
     from pyparrm_b200 import PARRM, _native, _sharding
@@ -901,7 +933,7 @@ def bench_search(engine, dist, world, rank, args):
     else:
         (tile,) = engine.prepare_tiles(data, [indices], 3.0)
     stream = torch.cuda.current_stream()
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     evaluate = lambda blk: engine.evaluate_device(tile, blk, bandwidth, 1.0, n_chans)  # noqa: E731
 
     def one_step():
@@ -920,6 +952,8 @@ def bench_search(engine, dist, world, rank, args):
     barrier(dist)
     seconds = max_over_ranks(dist, start.elapsed_time(stop) * 1e-3)
     assert errors.shape[0] == per_rank * world and np.isfinite(errors).all()
+    if args.dump_outputs and rank == 0:
+        dumped["find_period_errors"] = errors
 
     # FP64 FMA peak of this GPU, measured (no figure for it in MEASURED_PEAKS.json)
     sink = torch.zeros(8, dtype=torch.float64, device="cuda")
@@ -1015,10 +1049,21 @@ def bench_search(engine, dist, world, rank, args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50,
+                    help="timed passes of the headline, e2e, e2e_variants and find_period legs "
+                         "(the strong-scaling, standardise and power-capped figures time fixed "
+                         "counts of their own)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    if args.dump_outputs:  # an unwritable DIR fails here, not after the whole run
+        os.makedirs(args.dump_outputs, exist_ok=True)
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

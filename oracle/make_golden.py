@@ -14,11 +14,13 @@ re-implements its arithmetic):
   output, next to the shipped known answer ``matlab_filtered.npy``
   (examples/plot_use_parrm.py:43-45, 77-80, 135-141, 210-240).
 * ``synthetic_2x30000.npz``  seeded synthetic recording (random-index branch of
-  run 3): same captures, all three filter directions.
+  run 3): same captures, all three filter directions; the filtered outputs at the
+  columns ``oracle.golden_inputs.sample_columns`` picks.
 * ``ecog_lfp.npz``      bundled 2-channel ECoG/LFP recording: period + evaluations.
 * ``taps.npz``          tap offsets and default half-widths for a parameter sweep.
 * ``objective.npz``     ``_optimise_local`` values on seeded tiles.
-* ``filter_edges.npz``  short / ragged inputs (T < filter length, foreign data).
+* ``filter_edges.npz``  short / ragged inputs (T < filter length, foreign data); the inputs
+  are not stored, only their sha256 (``oracle.golden_inputs.filter_edges_inputs``).
 
 It also copies the four example ``.npy`` recordings into
 ``pyparrm_b200/data/example_data/`` (data files, not source) so that
@@ -27,7 +29,6 @@ It also copies the four example ``.npy`` recordings into
 
 from __future__ import annotations
 
-import hashlib
 import os
 import shutil
 import sys
@@ -41,14 +42,19 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 
 from oracle.ref_shim import import_reference  # noqa: E402
+from oracle.golden_inputs import (EDGE_FILTERS, EDGE_SHAPES, filter_edges_inputs,  # noqa: E402
+                                   sample_columns, sha)
 from pyparrm_b200.synthetic import make_recording  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 DATA_DST = os.path.join(ROOT, "pyparrm_b200", "data", "example_data")
 
 
-def sha(a: np.ndarray) -> str:
-    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+def store_filtered(out: dict, name: str, filtered: np.ndarray, taps: np.ndarray) -> None:
+    """Keep ``filtered`` at the columns ``sample_columns`` picks (``<name>_filtered_cols``)."""
+    cols = sample_columns(filtered.shape[1], taps)
+    out[f"{name}_filtered_cols"] = cols
+    out[f"{name}_filtered"] = np.ascontiguousarray(filtered[:, cols])
 
 
 def meta() -> dict:
@@ -154,11 +160,11 @@ def golden_synthetic(ref):
     for direction in ("both", "past", "future"):
         p.create_filter(filter_direction=direction)
         out[f"{direction}_taps"] = taps_of(p.filter)
-        out[f"{direction}_filtered"] = p.filter_data().copy()
+        store_filtered(out, direction, p.filter_data(), out[f"{direction}_taps"])
     out["default_half_width"] = np.int64(p._filter_half_width)
     p.create_filter(filter_half_width=2000, omit_n_samples=3, filter_direction="both")
     out["hw2000_taps"] = taps_of(p.filter)
-    out["hw2000_filtered"] = p.filter_data().copy()
+    store_filtered(out, "hw2000", p.filter_data(), out["hw2000_taps"])
     out["data_sha256"] = sha(data)
     out["recording"] = np.array([2, 30000, fs, fa, 1], dtype=np.int64)
     out.update(meta())
@@ -323,30 +329,22 @@ def golden_cfg2_objective(ref):
 
 def golden_filter_edges(ref):
     out = {}
-    rng = np.random.default_rng(11)
-    base = make_recording(2, 5000, 2000, 130, seed=9)
-    p = ref.PARRM(data=base, sampling_freq=2000, artefact_freq=130, verbose=False)
+    xs = filter_edges_inputs()
+    p = ref.PARRM(data=xs[0], sampling_freq=2000, artefact_freq=130, verbose=False)
     p._period = np.float64(2000 / 130 * (1 + 3e-6))
     case = 0
-    for hw, omit, direction, phw in (
-        (2000, 0, "both", None), (2000, 0, "past", None), (2000, 0, "future", None),
-        (300, 2, "both", 0.5), (2499, 10, "both", None),
-    ):
+    for hw, omit, direction, phw in EDGE_FILTERS:
         p.create_filter(filter_half_width=hw, omit_n_samples=omit,
                         filter_direction=direction, period_half_width=phw)
-        for shape in ((2, 5000), (1, 50), (3, 1), (1, 4001), (2, 2000), (1, 777)):
-            if shape == (2, 5000):
-                x = base
-            else:
-                x = rng.standard_normal(shape) + 10.0
-                out[f"case{case}_x"] = x
+        for _ in EDGE_SHAPES:
+            x = xs[case]
+            out[f"case{case}_x_sha256"] = sha(x)  # the tests regenerate x (oracle/golden_inputs.py)
             y = p.filter_data(x).copy()
             out[f"case{case}_y"] = y
             out[f"case{case}_taps"] = taps_of(p.filter)
             out[f"case{case}_hw"] = np.int64(hw)
             case += 1
     out["n_cases"] = np.int64(case)
-    out["base_x"] = base  # input of every case that stores no `_x`
     out.update(meta())
     np.savez_compressed(os.path.join(GOLDEN, "filter_edges.npz"), **out)
     print(f"filter_edges: {case} cases")
