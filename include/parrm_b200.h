@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PARRM_B200_ABI_VERSION 6
+#define PARRM_B200_ABI_VERSION 7
 
 typedef enum {
   PARRM_OK = 0,
@@ -253,6 +253,40 @@ int parrm_convert_f32_to_f64(const float* d_src, double* d_dst, int64_t n, void*
  * own width and are widened on the device. */
 int parrm_convert(const void* d_src, int src_type, void* d_dst, int dst_type, int64_t n,
                   void* stream);
+
+/* ------------------------------------------------------------------------
+ * Streaming filter: filter_data applied block by block as the recording is acquired (an
+ * online caller runs find_period / create_filter on a calibration segment, then filters every
+ * block the acquisition system delivers).  Concatenating every push's outputs and the closing
+ * push's gives exactly parrm_filter_apply with a PARRM_PLAN_GATHER plan on the concatenated
+ * recording, bit for bit: recording start and end edges and the non-finite rule included.
+ *
+ * Caller-owned state: d_ring of parrm_stream_ring_bytes() (the last span + max_chunk samples
+ * of every channel in the compute type, span = max(w_max, 0) - min(w_min, 0)), the ascending
+ * taps on the device (d_taps, n_taps, w_min = taps[0], w_max = taps[n_taps - 1]) and the
+ * position `pos`, the number of samples pushed before this block.
+ *
+ * parrm_stream_push enqueues ONE kernel that widens the block [n_chans, n] (storage type
+ * block_type, row stride ld_block, n <= max_chunk) into the ring and writes the outputs that
+ * are now final to d_out [n_chans, ld_out] in out_type:
+ *     open   (close = 0): outputs [max(0, pos - L), max(that, pos + n - L))
+ *     closing (close = 1): outputs [max(0, pos - L), pos + n), the recording ending at pos + n
+ * where L = max(0, -w_min) is the stream's latency: output t is final once sample t + L has
+ * arrived.  Under the reference's convolution y[t] reads x[t - w], so a "future" filter (w > 0)
+ * reads only earlier samples and has L = 0 -- it is the causal one -- while "past" and "both"
+ * need filter_half_width samples of look-ahead.  Work per push is O(n_chans * (n + span)).
+ * d_pos (may be NULL): device int64 the kernel reads the position from instead of `pos`, so
+ * that a push captured in a CUDA graph (H2D of a header + block -> kernel -> D2H) replays with
+ * a new position; the output count must then stay that of `pos` (it does for an open stream
+ * once pos >= L).  Errors: block longer than max_chunk, negative position, bad types.
+ * ---------------------------------------------------------------------- */
+size_t parrm_stream_ring_bytes(int64_t n_chans, const int32_t* h_taps, int32_t n_taps,
+                               int64_t max_chunk, int dtype);
+int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const int32_t* d_taps,
+                      int32_t n_taps, int32_t w_min, int32_t w_max, const void* d_block,
+                      int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
+                      int64_t ld_out, int64_t pos, const int64_t* d_pos, int close, int dtype,
+                      void* stream);
 
 /* ------------------------------------------------------------------------
  * Device-resident Nelder-Mead: the scipy.optimize.fmin refinements of find_period

@@ -15,7 +15,7 @@ from __future__ import annotations
 import ctypes
 import os
 import threading
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 
 import numpy as np
 
@@ -102,6 +102,28 @@ class SearchTile:
         import torch
 
         return _native.F32 if self.y.dtype == torch.float32 else _native.F64
+
+
+@dataclass(eq=False)
+class _StreamState:
+    """Device state of one streaming filter (``DeviceEngine.stream_open``)."""
+
+    taps: np.ndarray
+    d_taps: object
+    max_chunk: int
+    code: int           # compute type of the ring and the kernel
+    latency: int
+    device: object
+    stream: object      # torch.cuda.Stream every push of this stream runs on
+    n_chans: int | None = None
+    on_device: bool | None = None
+    ring: object = None
+    d_in: object = None       # [header | block] as the kernel reads it
+    stage_in: object = None   # pinned twin of d_in
+    d_out: object = None
+    stage_out: object = None
+    graphs: dict = field(default_factory=dict)   # push shape -> captured CUDA graph
+    seen: set = field(default_factory=set)       # push shapes run once eagerly
 
 
 class DeviceEngine:
@@ -849,6 +871,161 @@ class DeviceEngine:
             for k in range(_N_SLOTS):
                 drain(k)
             self.s_out.synchronize()
+        return out
+
+    # ------------------------------------------------------------- streaming
+    _STREAM_HEADER = 64      # bytes before the block in the staging buffers: the position
+    _STREAM_GRAPHS = 4       # captured push shapes kept per stream
+
+    def stream_open(self, taps: np.ndarray, max_chunk: int, precision: str = "fp64"):
+        """State of one streaming filter (:mod:`pyparrm_b200._stream`): taps on the device, a
+        CUDA stream of its own, and -- from the first push, which fixes the channel count -- the
+        ring of the last ``span + max_chunk`` samples per channel and pinned in/out staging.
+        Two streams never share any of it."""
+        t = self.torch
+        taps = np.ascontiguousarray(taps, dtype=np.int32)
+        with self._lock, t.cuda.device(self.device):
+            return _StreamState(
+                taps=taps, d_taps=t.from_numpy(taps).to(self.device), max_chunk=int(max_chunk),
+                code=_native.F32 if precision == "fp32" else _native.F64,
+                latency=max(0, -int(taps[0])), device=self.device,
+                stream=t.cuda.Stream(device=self.device))
+
+    def _stream_buffers(self, st, n_chans: int, in_bytes: int, out_bytes: int) -> None:
+        """Ring at the first push; staging grown to the largest push (captured graphs hold the
+        old pointers, so growing drops them)."""
+        t = self.torch
+        if st.ring is None:
+            nbytes = lib.parrm_stream_ring_bytes(n_chans, _vp(st.taps.ctypes.data),
+                                                 int(st.taps.shape[0]), st.max_chunk, st.code)
+            if nbytes == 0:
+                check(1, "parrm_stream_ring_bytes")
+            st.ring = self._empty(nbytes, t.uint8)
+            st.n_chans = n_chans
+        in_bytes += self._STREAM_HEADER
+        if st.d_in is None or st.d_in.numel() < in_bytes:
+            st.d_in = self._empty(in_bytes, t.uint8)
+            st.stage_in = t.empty(in_bytes, dtype=t.uint8, pin_memory=True)
+            st.graphs.clear()
+        if st.d_out is None or st.d_out.numel() < max(out_bytes, 16):
+            st.d_out = self._empty(max(out_bytes, 16), t.uint8)
+            st.stage_out = t.empty(max(out_bytes, 16), dtype=t.uint8, pin_memory=True)
+            st.graphs.clear()
+
+    def _stream_launch(self, st, d_block, block_code, ld_block, n, d_out, out_code, k, pos,
+                       d_pos, close, sp) -> None:
+        w_min, w_max = int(st.taps[0]), int(st.taps[-1])
+        check(lib.parrm_stream_push(
+            _vp(st.ring.data_ptr()), st.n_chans, st.max_chunk, _vp(st.d_taps.data_ptr()),
+            int(st.taps.shape[0]), w_min, w_max, _vp(d_block), block_code, ld_block, n,
+            _vp(d_out), out_code, max(k, 1), pos, d_pos, int(close), st.code, sp),
+            "parrm_stream_push")
+
+    def stream_push(self, st, block, pos: int, close: bool, out_dtype=None, graphs: bool = False):
+        """One push (``block`` None: nothing new, the closing push): returns the outputs it makes
+        final, ``_stream.output_range``.  NumPy blocks go through the stream's pinned staging
+        (H2D, one kernel, D2H, on the stream's own CUDA stream); with ``graphs``, a push of the
+        same shape as an earlier one, on an open stream past its latency, is captured once and
+        then replayed as one CUDA graph that reads the position from a header copied up with
+        the block.  CUDA blocks are read where they lie and a CUDA tensor comes back."""
+        from ._stream import output_range
+
+        t = self.torch
+        with self._lock, t.cuda.device(self.device):
+            if st.on_device is None:
+                st.on_device = block is not None and not isinstance(block, np.ndarray)
+            if st.on_device:
+                return self._stream_push_device(st, block, pos, close, output_range)
+            if block is None:
+                block = np.zeros((st.n_chans, 0), dtype=np.float64)
+            data, in_code = self._as_storage_array(block)
+            n_chans, n = data.shape
+            out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
+            out_code = _native.F64 if out_np == np.float64 else _native.F32
+            lo, hi = output_range(pos, n, st.latency, close)
+            k = hi - lo
+            in_bytes, out_bytes = data.nbytes, n_chans * k * out_np.itemsize
+            self._stream_buffers(st, n_chans, in_bytes, out_bytes)
+            hdr = self._STREAM_HEADER
+            d_in, h_in = st.d_in.data_ptr(), st.stage_in.data_ptr()
+            d_out, h_out = st.d_out.data_ptr(), st.stage_out.data_ptr()
+            if in_bytes:
+                _threaded_memmove(h_in + hdr, data.ctypes.data, in_bytes)
+            sp = self._stream_ptr(st.stream)
+            key = (n_chans, n, in_code, out_code)
+            replayable = graphs and not close and pos >= st.latency and n > 0
+            if replayable and (key in st.graphs or key in st.seen):
+                st.stage_in[:8].numpy().view(np.int64)[0] = pos
+                graph = st.graphs.get(key)
+                if graph is None:
+                    graph = self._stream_capture(st, key, data.shape, in_code, out_code, k, pos)
+                with t.cuda.stream(st.stream):
+                    graph.replay()
+                self.launches += 1
+                self.graph_kernels += 1
+            else:
+                check(lib.parrm_copy_h2d_async(_vp(d_in + hdr), _vp(h_in + hdr), in_bytes, sp),
+                      "H2D copy")
+                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos, None,
+                                    close, sp)
+                self.launches += 1
+                check(lib.parrm_copy_d2h_async(_vp(h_out), _vp(d_out), out_bytes, sp), "D2H copy")
+                if replayable:
+                    st.seen.add(key)
+            st.stream.synchronize()
+            view = st.stage_out[:out_bytes].numpy().view(out_np).reshape(n_chans, k)
+            return view.copy()
+
+    def _stream_capture(self, st, key, shape, in_code, out_code, k, pos):
+        """Capture H2D (header + block) -> kernel -> D2H of a push shape as one CUDA graph."""
+        t = self.torch
+        n_chans, n = shape
+        es_in = {_native.F64: 8, _native.F32: 4, _native.I16: 2, _native.I32: 4}[in_code]
+        es_out = 8 if out_code == _native.F64 else 4
+        hdr = self._STREAM_HEADER
+        d_in, h_in = st.d_in.data_ptr(), st.stage_in.data_ptr()
+        d_out, h_out = st.d_out.data_ptr(), st.stage_out.data_ptr()
+        graph = t.cuda.CUDAGraph()
+        with t.cuda.stream(st.stream):
+            sp = self._stream_ptr(st.stream)
+            graph.capture_begin(capture_error_mode="thread_local")
+            try:
+                check(lib.parrm_copy_h2d_async(_vp(d_in), _vp(h_in), hdr + n_chans * n * es_in, sp),
+                      "H2D copy")
+                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos,
+                                    _vp(d_in), False, sp)
+                check(lib.parrm_copy_d2h_async(_vp(h_out), _vp(d_out), n_chans * k * es_out, sp),
+                      "D2H copy")
+            finally:
+                graph.capture_end()
+        if len(st.graphs) >= self._STREAM_GRAPHS:
+            st.graphs.pop(next(iter(st.graphs)))
+        st.graphs[key] = graph
+        return graph
+
+    _TORCH_STORAGE = {"torch.float64": _native.F64, "torch.float32": _native.F32,
+                      "torch.int16": _native.I16, "torch.int32": _native.I32}
+
+    def _stream_push_device(self, st, block, pos, close, output_range):
+        t = self.torch
+        comp = t.float32 if st.code == _native.F32 else t.float64
+        if block is None:
+            block = t.empty((st.n_chans, 0), dtype=comp, device=self.device)
+        code = self._TORCH_STORAGE.get(str(block.dtype))
+        if code is None:
+            block, code = block.to(t.float64), _native.F64
+        if block.stride(1) != 1 and block.shape[1] > 1:
+            block = block.contiguous()
+        n_chans, n = block.shape
+        lo, hi = output_range(pos, n, st.latency, close)
+        self._stream_buffers(st, n_chans, 0, 0)
+        out = t.empty((n_chans, hi - lo), dtype=comp, device=self.device)
+        current = t.cuda.current_stream()
+        st.stream.wait_stream(current)
+        self._stream_launch(st, block.data_ptr(), code, max(block.stride(0), n), n, out.data_ptr(),
+                            st.code, hi - lo, pos, None, close, self._stream_ptr(st.stream))
+        self.launches += 1
+        current.wait_stream(st.stream)
         return out
 
     # Results are handed to the caller in page-locked memory (direct D2H, no staging copy) up

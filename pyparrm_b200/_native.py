@@ -20,7 +20,7 @@ DIR_BOTH, DIR_PAST, DIR_FUTURE = 0, 1, 2
 DIRECTIONS = {"both": DIR_BOTH, "past": DIR_PAST, "future": DIR_FUTURE}
 MAX_BANDWIDTH = 23
 NM_STATE_BYTES = 88
-ABI_VERSION = 6
+ABI_VERSION = 7
 PLAN_AUTO, PLAN_GATHER, PLAN_COMB = 0, 1, 2
 KERNEL_AUTO, KERNEL_GATHER, KERNEL_SPECIALISED = 0, 1, 3
 
@@ -122,6 +122,12 @@ SIGNATURES = {
     "parrm_periodogram": (
         c_int,
         [c_void_p, c_int64, c_int64, c_int64, c_int, c_int64, c_double, c_void_p, c_int64, c_void_p],
+    ),
+    "parrm_stream_ring_bytes": (c_size_t, [c_int64, c_void_p, c_int32, c_int64, c_int]),
+    "parrm_stream_push": (
+        c_int,
+        [c_void_p, c_int64, c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int,
+         c_int64, c_int64, c_void_p, c_int, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p],
     ),
     "parrm_fp64_fma_burn": (c_int, [c_int64, c_void_p, POINTER(c_double), c_void_p]),
 }

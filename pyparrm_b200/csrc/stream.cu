@@ -1,0 +1,325 @@
+// Streaming filter: filter_data applied block by block as a recording is acquired.
+//
+// State per stream (all caller-owned device memory):
+//   ring[c * R + (t mod R)]  the last R samples of every channel, in the compute type, with
+//                            R = span + max_chunk,  span = max(w_max, 0) - min(w_min, 0);
+//   taps                     ascending offsets, as parrm_build_taps produces them;
+//   pos                      samples pushed before this block (a host argument, or a device
+//                            int64 so that a captured CUDA graph can replay with a new position).
+//
+// One launch per push.  The block holds samples [pos, pos + n) in its storage type.  Output t
+// reads samples t - w for the taps w; it is final once sample t + L exists, L = max(0, -w_min),
+// so while the stream is open a push produces outputs [max(0, pos - L), pos + n - L) and the
+// closing push the rest, up to pos + n, with the recording-end edge.  Treating the recording as
+// ending at pos + n is exact for the open outputs too: none of their taps reaches past it.
+//
+// Every CTA reads samples >= pos from the incoming block and older ones from the ring, and
+// writes only its own slice of the block into the ring.  The oldest sample any output of this
+// launch reads is pos - span, and R >= span + n, so the slots written here ((pos .. pos+n-1)
+// mod R) are never slots read here: no grid-wide barrier is needed.  Work and traffic per push
+// are O(channels x (n + span)), independent of how much has been pushed.
+//
+// Arithmetic: the same floating-point operations in the same order as the gather kernels of
+// filter.cu (ascending taps, sequential adds, acc / n_taps in the interior, acc / n_in at the
+// edges, finite_or_zero(x - mean)), so a streamed recording is bit-equal to filter_data with
+// a gather plan on the whole of it.  Widening from the storage type is parrm_convert's
+// static_cast, narrowing to the output type likewise.
+#include <limits.h>
+
+#include "common.cuh"
+
+namespace parrm {
+
+constexpr int kStreamThreads = 256;
+constexpr int kStreamOutPerThread = 4;
+constexpr int kStreamSmemBudget = 200 * 1024;
+
+__host__ __device__ inline int round16s(int bytes) { return (bytes + 15) & ~15; }
+
+template <typename T>
+struct StreamArgs {
+  T* ring;
+  const int32_t* taps;
+  const void* block;
+  void* out;
+  const int64_t* d_pos;
+  int64_t ring_len, ld_block, n, ld_out, pos;
+  int32_t n_taps, w_lo, w_hi, tile;
+  int32_t block_type, out_type, close;
+};
+
+template <typename T>
+__device__ __forceinline__ T finite_or_zero_s(T y) {
+  return isfinite(y) ? y : T(0);
+}
+
+template <typename T>
+__device__ __forceinline__ T load_block(const void* b, int type, int64_t i) {
+  switch (type) {
+    case PARRM_F64: return static_cast<T>(static_cast<const double*>(b)[i]);
+    case PARRM_F32: return static_cast<T>(static_cast<const float*>(b)[i]);
+    case PARRM_I16: return static_cast<T>(static_cast<const int16_t*>(b)[i]);
+    default: return static_cast<T>(static_cast<const int32_t*>(b)[i]);
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ void store_out(void* o, int type, int64_t i, T y) {
+  if (type == PARRM_F64)
+    static_cast<double*>(o)[i] = static_cast<double>(y);
+  else
+    static_cast<float*>(o)[i] = static_cast<float>(y);
+}
+
+// Position, output range and recording end of this push (identical in every CTA).
+struct StreamRange {
+  int64_t pos, out_lo, out_hi, n_total;
+};
+
+template <typename T>
+__device__ __forceinline__ StreamRange stream_range(const StreamArgs<T>& a) {
+  StreamRange r;
+  r.pos = a.d_pos ? *a.d_pos : a.pos;
+  const int64_t lat = -int64_t(a.w_lo);
+  r.out_lo = max(int64_t(0), r.pos - lat);
+  r.n_total = r.pos + a.n;
+  r.out_hi = a.close ? r.n_total : max(r.out_lo, r.n_total - lat);
+  return r;
+}
+
+// This CTA's slice [x * tile, (x + 1) * tile) of the block, widened, into the ring.
+template <typename T>
+__device__ __forceinline__ void block_to_ring(const StreamArgs<T>& a, const StreamRange& r,
+                                              int64_t chan) {
+  const int64_t b0 = int64_t(blockIdx.x) * a.tile;
+  const int64_t b1 = min(b0 + a.tile, a.n);
+  if (b0 >= b1) return;
+  T* ring = a.ring + chan * a.ring_len;
+  const int64_t base = (r.pos + b0) % a.ring_len;  // the slice is shorter than R: one wrap at most
+  for (int64_t i = b0 + threadIdx.x; i < b1; i += kStreamThreads) {
+    int64_t j = base + (i - b0);
+    if (j >= a.ring_len) j -= a.ring_len;
+    ring[j] = load_block<T>(a.block, a.block_type, chan * a.ld_block + i);
+  }
+}
+
+// ---- shared-memory gather: one output tile + its tap window per CTA ------------------------
+template <typename T>
+__global__ void __launch_bounds__(kStreamThreads)
+stream_gather_smem_kernel(const StreamArgs<T> a) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  int32_t* s_taps = reinterpret_cast<int32_t*>(smem_raw);
+  T* s_win = reinterpret_cast<T*>(smem_raw + round16s(a.n_taps * 4));
+  const int tid = threadIdx.x;
+  const int64_t chan = blockIdx.y;
+  const StreamRange r = stream_range(a);
+  block_to_ring(a, r, chan);
+
+  const int64_t tile_t0 = r.out_lo + int64_t(blockIdx.x) * a.tile;
+  if (tile_t0 >= r.out_hi) return;
+  const int n_tile = int(min(int64_t(a.tile), r.out_hi - tile_t0));
+  const int64_t g_lo = tile_t0 - a.w_hi;              // window of sample times in s_win
+  const int64_t g_hi = tile_t0 + n_tile - a.w_lo;
+  const int64_t v_lo = max(g_lo, int64_t(0));
+  const int64_t v_mid = max(v_lo, min(g_hi, r.pos));  // [v_lo, v_mid) from the ring
+  const int64_t v_hi = min(g_hi, r.n_total);          // [v_mid, v_hi) from the block
+  const T* ring = a.ring + chan * a.ring_len;
+  const int64_t ring0 = v_lo % a.ring_len;            // at most span samples: one wrap at most
+
+  for (int i = tid; i < a.n_taps; i += kStreamThreads) s_taps[i] = a.taps[i];
+  for (int i = tid; i < int(g_hi - g_lo); i += kStreamThreads) {
+    const int64_t g = g_lo + i;
+    T v = T(0);
+    if (g >= v_lo && g < v_mid) {
+      int64_t j = ring0 + (g - v_lo);
+      if (j >= a.ring_len) j -= a.ring_len;
+      v = ring[j];
+    } else if (g >= v_mid && g < v_hi) {
+      v = load_block<T>(a.block, a.block_type, chan * a.ld_block + (g - r.pos));
+    }
+    s_win[i] = v;
+  }
+  __syncthreads();
+
+  const T* s_c = s_win + a.w_hi;  // s_c[i] = sample at tile_t0 + i
+  const int64_t o0 = chan * a.ld_out + (tile_t0 - r.out_lo);
+  const bool interior = (g_lo >= 0) && (g_hi <= r.n_total);
+  const int n_taps = a.n_taps;
+
+  if (interior) {
+    const T inv_scale = T(n_taps);
+    for (int i0 = tid; i0 < n_tile; i0 += kStreamThreads * kStreamOutPerThread) {
+      T acc[kStreamOutPerThread];
+#pragma unroll
+      for (int q = 0; q < kStreamOutPerThread; ++q) acc[q] = T(0);
+      int idx[kStreamOutPerThread];
+#pragma unroll
+      for (int q = 0; q < kStreamOutPerThread; ++q)
+        idx[q] = min(i0 + q * kStreamThreads, n_tile - 1);
+#pragma unroll 4
+      for (int k = 0; k < n_taps; ++k) {
+        const int w = s_taps[k];
+#pragma unroll
+        for (int q = 0; q < kStreamOutPerThread; ++q) acc[q] += s_c[idx[q] - w];
+      }
+#pragma unroll
+      for (int q = 0; q < kStreamOutPerThread; ++q) {
+        const int i = i0 + q * kStreamThreads;
+        if (i < n_tile)
+          store_out(a.out, a.out_type, o0 + i, finite_or_zero_s(s_c[i] - acc[q] / inv_scale));
+      }
+    }
+  } else {
+    for (int i = tid; i < n_tile; i += kStreamThreads) {
+      const int64_t t = tile_t0 + i;
+      T acc = T(0);
+      int n_in = 0;
+      for (int k = 0; k < n_taps; ++k) {
+        const int w = s_taps[k];
+        const int64_t src = t - w;
+        if (src >= 0 && src < r.n_total) {
+          acc += s_c[i - w];
+          ++n_in;
+        }
+      }
+      store_out(a.out, a.out_type, o0 + i,
+                n_in > 0 ? finite_or_zero_s(s_c[i] - acc / T(n_in)) : T(0));
+    }
+  }
+}
+
+// ---- global-memory gather: tap windows too wide for shared memory -------------------------
+// The ring of such a stream is read from L2 (384 channels x a 4 k-sample span x 8 B ~ 12 MB).
+template <typename T>
+__global__ void __launch_bounds__(kStreamThreads)
+stream_gather_global_kernel(const StreamArgs<T> a) {
+  const int64_t chan = blockIdx.y;
+  const StreamRange r = stream_range(a);
+  block_to_ring(a, r, chan);
+  const int64_t t = r.out_lo + int64_t(blockIdx.x) * a.tile + threadIdx.x;
+  if (t >= r.out_hi) return;
+  const T* ring = a.ring + chan * a.ring_len;
+  const int64_t blk = chan * a.ld_block - r.pos;  // block element of sample s >= pos: blk + s
+  T acc = T(0);
+  int n_in = 0;
+  for (int k = 0; k < a.n_taps; ++k) {
+    const int64_t src = t - a.taps[k];
+    if (src >= 0 && src < r.n_total) {
+      acc += src >= r.pos ? load_block<T>(a.block, a.block_type, blk + src)
+                          : ring[src % a.ring_len];
+      ++n_in;
+    }
+  }
+  const T x = t >= r.pos ? load_block<T>(a.block, a.block_type, blk + t) : ring[t % a.ring_len];
+  store_out(a.out, a.out_type, chan * a.ld_out + (t - r.out_lo),
+            n_in > 0 ? finite_or_zero_s(x - acc / T(n_in)) : T(0));
+}
+
+static int64_t stream_span(int32_t w_min, int32_t w_max) {
+  return int64_t(w_max > 0 ? w_max : 0) - int64_t(w_min < 0 ? w_min : 0);
+}
+
+template <typename T>
+int launch_stream(StreamArgs<T> a, int64_t n_chans, int64_t n_out_max, cudaStream_t stream) {
+  const int64_t span = int64_t(a.w_hi) - a.w_lo;
+  const int64_t fixed = round16s(a.n_taps * 4);
+  const int64_t es = int64_t(sizeof(T));
+  if (fixed + (kStreamThreads + span) * es > kStreamSmemBudget) {
+    a.tile = kStreamThreads;
+    dim3 grid(unsigned(ceil_div(n_out_max, a.tile)), unsigned(n_chans));
+    stream_gather_global_kernel<T><<<grid, kStreamThreads, 0, stream>>>(a);
+    PARRM_LAUNCH_OK("stream_gather_global_kernel");
+    return PARRM_OK;
+  }
+  // Tiles of 256..4096 outputs: enough CTAs to cover the GPU twice when the push allows it,
+  // no more outputs per CTA than the push has, and the window within the shared-memory budget.
+  const int64_t want = ceil_div(n_out_max * n_chans, 2 * int64_t(kNumSMs));
+  int64_t tile = ceil_div(max64(want, 1), kStreamThreads) * kStreamThreads;
+  tile = min64(min64(tile, 4096), ceil_div(n_out_max, kStreamThreads) * kStreamThreads);
+  while (tile > kStreamThreads && fixed + (tile + span) * es > kStreamSmemBudget)
+    tile -= kStreamThreads;
+  a.tile = int32_t(tile);
+  const size_t smem = size_t(fixed + (tile + span) * es);
+  PARRM_CUDA_OK(cudaFuncSetAttribute(stream_gather_smem_kernel<T>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
+  dim3 grid(unsigned(ceil_div(n_out_max, tile)), unsigned(n_chans));
+  stream_gather_smem_kernel<T><<<grid, kStreamThreads, smem, stream>>>(a);
+  PARRM_LAUNCH_OK("stream_gather_smem_kernel");
+  return PARRM_OK;
+}
+
+}  // namespace parrm
+
+extern "C" {
+
+size_t parrm_stream_ring_bytes(int64_t n_chans, const int32_t* h_taps, int32_t n_taps,
+                               int64_t max_chunk, int dtype) {
+  using namespace parrm;
+  if (h_taps == nullptr || n_taps < 1 || n_chans < 1 || max_chunk < 1 ||
+      (dtype != PARRM_F64 && dtype != PARRM_F32)) {
+    set_error("parrm_stream_ring_bytes: need taps, channels >= 1, max_chunk >= 1 and a "
+              "float64 / float32 compute type");
+    return 0;
+  }
+  for (int32_t i = 1; i < n_taps; ++i) {
+    if (h_taps[i] <= h_taps[i - 1]) {
+      set_error("parrm_stream_ring_bytes: taps must be strictly ascending");
+      return 0;
+    }
+  }
+  const int64_t ring_len = stream_span(h_taps[0], h_taps[n_taps - 1]) + max_chunk;
+  return size_t(n_chans) * size_t(ring_len) * (dtype == PARRM_F64 ? 8 : 4);
+}
+
+int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const int32_t* d_taps,
+                      int32_t n_taps, int32_t w_min, int32_t w_max, const void* d_block,
+                      int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
+                      int64_t ld_out, int64_t pos, const int64_t* d_pos, int close, int dtype,
+                      void* stream) {
+  PARRM_NVTX("parrm_stream_push");
+  using namespace parrm;
+  PARRM_REQUIRE(dtype == PARRM_F64 || dtype == PARRM_F32, "parrm_stream_push: bad dtype %d", dtype);
+  PARRM_REQUIRE(out_type == PARRM_F64 || out_type == PARRM_F32,
+                "parrm_stream_push: bad output type %d", out_type);
+  PARRM_REQUIRE(block_type == PARRM_F64 || block_type == PARRM_F32 || block_type == PARRM_I16 ||
+                    block_type == PARRM_I32,
+                "parrm_stream_push: unknown block storage type %d", block_type);
+  PARRM_REQUIRE(n_chans >= 1 && n_chans <= 65535, "parrm_stream_push: 1..65535 channels, got %lld",
+                (long long)n_chans);
+  PARRM_REQUIRE(n_taps >= 1 && w_min <= w_max, "parrm_stream_push: empty or unordered tap list");
+  PARRM_REQUIRE(max_chunk >= 1, "parrm_stream_push: max_chunk must be >= 1");
+  PARRM_REQUIRE(n >= 0 && n <= max_chunk,
+                "parrm_stream_push: block of %lld samples is longer than the ring allows "
+                "(max_chunk %lld)", (long long)n, (long long)max_chunk);
+  PARRM_REQUIRE(pos >= 0, "parrm_stream_push: position %lld goes backwards past the stream start",
+                (long long)pos);
+  PARRM_REQUIRE(pos <= INT64_MAX / 2, "parrm_stream_push: position %lld out of range",
+                (long long)pos);
+  PARRM_REQUIRE(d_ring != nullptr && d_taps != nullptr, "parrm_stream_push: null ring or taps");
+  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
+  const int64_t out_lo = pos - lat > 0 ? pos - lat : 0;
+  const int64_t out_hi = close ? pos + n : (pos + n - lat > out_lo ? pos + n - lat : out_lo);
+  const int64_t n_out_max = n + (close ? lat : 0);  // grid extent; independent of pos
+  if (n == 0 && out_hi == out_lo) return PARRM_OK;
+  PARRM_REQUIRE(n == 0 || (d_block != nullptr && ld_block >= n),
+                "parrm_stream_push: null block or row stride %lld < %lld", (long long)ld_block,
+                (long long)n);
+  PARRM_REQUIRE(out_hi == out_lo || (d_out != nullptr && ld_out >= out_hi - out_lo),
+                "parrm_stream_push: null output or row stride %lld < %lld outputs",
+                (long long)ld_out, (long long)(out_hi - out_lo));
+  const int64_t ring_len = stream_span(w_min, w_max) + max_chunk;
+  const int32_t w_lo = w_min < 0 ? w_min : 0, w_hi = w_max > 0 ? w_max : 0;
+  cudaStream_t s = as_stream(stream);
+  if (dtype == PARRM_F64) {
+    StreamArgs<double> a{static_cast<double*>(d_ring), d_taps, d_block, d_out, d_pos, ring_len,
+                         ld_block, n, ld_out, pos, n_taps, w_lo, w_hi, 0, block_type, out_type,
+                         close ? 1 : 0};
+    return launch_stream<double>(a, n_chans, n_out_max, s);
+  }
+  StreamArgs<float> a{static_cast<float*>(d_ring), d_taps, d_block, d_out, d_pos, ring_len,
+                      ld_block, n, ld_out, pos, n_taps, w_lo, w_hi, 0, block_type, out_type,
+                      close ? 1 : 0};
+  return launch_stream<float>(a, n_chans, n_out_max, s);
+}
+
+}  // extern "C"

@@ -533,8 +533,7 @@ class PARRM:
                 "The filter has not yet been created. The `create_filter` method must "
                 "be called first."
             )
-        half_width = (self._filter.shape[0] - 1) // 2
-        taps = (np.flatnonzero(self._filter < 0) - half_width).astype(np.int32)
+        taps = self._tap_offsets()
         engine = _engine.get_engine()
         if _is_device_tensor(data):
             # additive overload (SURVEY 8(f).2): a CUDA tensor [channels, times] (float64 or
@@ -565,6 +564,50 @@ class PARRM:
         if self._verbose:
             print("    ... Data filtered\n")
         return self._filtered_data
+
+    def _tap_offsets(self) -> np.ndarray:
+        """Ascending offsets ``w`` of the filter's taps (``y[t]`` reads ``x[t - w]``)."""
+        half_width = (self._filter.shape[0] - 1) // 2
+        return (np.flatnonzero(self._filter < 0) - half_width).astype(np.int32)
+
+    def filter_stream(self, *, max_chunk=1 << 16, out_dtype=None, graphs=False):
+        """Filter a recording block by block as it is acquired (additive).
+
+        Returns a :class:`pyparrm_b200._stream.FilterStream` holding a snapshot of this
+        object's filter and precision (a later ``create_filter()`` does not affect it)::
+
+            parrm.find_period(); parrm.create_filter(filter_direction="future")
+            stream = parrm.filter_stream()
+            for block in acquisition:     # [channels, n] NumPy array or CUDA tensor
+                y = stream.push(block)    # [channels, k]: every output that is now final
+            tail = stream.close()         # the last `stream.latency` outputs
+
+        The pushes and ``close()`` concatenate to exactly ``filter_data()`` of the concatenated
+        recording.  Output ``t`` is final once sample ``t + stream.latency`` has arrived;
+        ``latency = max(0, -min(taps))`` is 0 for ``filter_direction="future"``, the causal
+        direction (``y[t]`` reads ``x[t - w]``, and its taps ``w`` are positive), and
+        ``filter_half_width`` at most for ``"past"`` and ``"both"``.
+
+        ``max_chunk``: the longest push the device ring is sized for (longer pushes are split
+        on the host).  ``out_dtype``: float64 (default) or float32 NumPy results; CUDA-tensor
+        pushes return CUDA tensors in the compute type.  ``graphs=True`` replays NumPy pushes of a
+        repeated shape as one CUDA graph (H2D, kernel, D2H); the results are the same bit for
+        bit, but on a B200 it measured 8-18 us slower per push than the default separate
+        launches (profiles/r3/stream_latency.txt).  Not available under ``enable_sharding()``."""
+        if self._filter is None:
+            raise ValueError(
+                "The filter has not yet been created. The `create_filter` method must "
+                "be called first."
+            )
+        if _sharding.active():
+            raise NotImplementedError(
+                "filter_stream() does not shard: a stream runs on this rank's GPU only. Call "
+                "disable_sharding() first, or filter whole recordings with filter_data()."
+            )
+        from ._stream import FilterStream
+
+        return FilterStream(_engine.get_engine(), self._tap_offsets(), self._precision,
+                            max_chunk=max_chunk, out_dtype=out_dtype, graphs=graphs)
 
     def filter_sweep(self, parameter_sets, data=None):
         """Filter with many parameter sets at once (additive; SURVEY 8(f).4).
