@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PARRM_B200_ABI_VERSION 7
+#define PARRM_B200_ABI_VERSION 8
 
 typedef enum {
   PARRM_OK = 0,
@@ -287,6 +287,33 @@ int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const in
                       int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
                       int64_t ld_out, int64_t pos, const int64_t* d_pos, int close, int dtype,
                       void* stream);
+
+/* parrm_stream_push_at: the same kernel with the ring length and the first output passed
+ * explicitly, for a stream whose taps were switched while it was open (a re-calibrated
+ * filter).  d_ring holds the last ring_len samples of every channel ([n_chans, ring_len], any
+ * ring_len the caller allocated); the push writes outputs [out_lo, out_hi) to d_out, with
+ *     out_hi = close ? pos + n : max(out_lo, pos + n - L),   L = max(0, -w_min),
+ * so after a switch to a smaller latency a push can emit more than n outputs, and after a
+ * switch to a larger one none.  With one tap set, out_lo = max(0, pos - L) and
+ * ring_len = span + max_chunk give exactly parrm_stream_push.  Requirements (else
+ * PARRM_ERR_INVALID_ARGUMENT): 0 <= out_lo <= pos, n >= 0, and the ring invariant
+ *     pos + n - max(0, out_lo - max(w_max, 0)) <= ring_len:
+ * every sample the launch reads is still in the ring, and no slot it writes is read in it.
+ * d_hdr (may be NULL): device int64 {pos, out_lo} read instead of the host values, so that a
+ * captured CUDA graph replays with new positions; the output count must stay the one the host
+ * arguments give.  Same arithmetic, bit for bit, as parrm_stream_push. */
+int parrm_stream_push_at(void* d_ring, int64_t ring_len, int64_t n_chans, const int32_t* d_taps,
+                         int32_t n_taps, int32_t w_min, int32_t w_max, const void* d_block,
+                         int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
+                         int64_t ld_out, int64_t pos, int64_t out_lo, const int64_t* d_hdr,
+                         int close, int dtype, void* stream);
+
+/* parrm_stream_window: copy the last n samples of a stream's ring (ring_len slots per channel,
+ * pos samples pushed) to d_dst: d_dst[c * ld_dst + i] = sample pos - n + i of channel c, in the
+ * ring's compute type.  Requires 1 <= n <= min(pos, ring_len) and ld_dst >= n.  At most two
+ * strided device-to-device copies on `stream` (the window wraps the ring at most once). */
+int parrm_stream_window(const void* d_ring, int64_t ring_len, int64_t n_chans, int64_t pos,
+                        int64_t n, void* d_dst, int64_t ld_dst, int dtype, void* stream);
 
 /* ------------------------------------------------------------------------
  * Device-resident Nelder-Mead: the scipy.optimize.fmin refinements of find_period

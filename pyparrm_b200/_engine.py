@@ -115,6 +115,7 @@ class _StreamState:
     latency: int
     device: object
     stream: object      # torch.cuda.Stream every push of this stream runs on
+    ring_len: int       # samples per channel: max(span of the first taps, history) + max_chunk
     n_chans: int | None = None
     on_device: bool | None = None
     ring: object = None
@@ -124,6 +125,7 @@ class _StreamState:
     stage_out: object = None
     graphs: dict = field(default_factory=dict)   # push shape -> captured CUDA graph
     seen: set = field(default_factory=set)       # push shapes run once eagerly
+    lock: object = field(default_factory=threading.Lock)  # this stream's state, not the engine's
 
 
 class DeviceEngine:
@@ -145,6 +147,7 @@ class DeviceEngine:
             self.s_run = torch.cuda.Stream()
             self.s_out = torch.cuda.Stream()
         self._lock = threading.RLock()
+        self._count_lock = threading.Lock()  # the counters below; streams run outside _lock
         self._ring = None          # (key, slots)
         self._stage_in = None      # pinned staging for pageable inputs
         self._stage_out = None
@@ -155,6 +158,11 @@ class DeviceEngine:
         self.last_filter_kernel = ""
 
     # ------------------------------------------------------------------ helpers
+    def _count(self, launches: int = 0, graph_kernels: int = 0) -> None:
+        with self._count_lock:
+            self.launches += launches
+            self.graph_kernels += graph_kernels
+
     def _stream_ptr(self, stream) -> ctypes.c_void_p:
         return _vp(stream.cuda_stream)
 
@@ -209,9 +217,14 @@ class DeviceEngine:
         reads (parrm.py:589-591), for every run's index set at once.
         """
         t = self.torch
-        data, dtype_code = self._as_float_array(data, allow_f32=True)
+        on_device = not isinstance(data, np.ndarray)
+        if on_device:
+            data, dtype_code = self._device_recording(data)
+            elem = data.element_size()
+        else:
+            data, dtype_code = self._as_float_array(data, allow_f32=True)
+            elem = data.dtype.itemsize
         n_chans, n_samples = data.shape
-        elem = data.dtype.itemsize
         with self._lock, t.cuda.device(self.device):
             tiles = []
             for idx in index_sets:
@@ -230,6 +243,9 @@ class DeviceEngine:
                 )
             rows = max(1, _SEARCH_CHUNK_BYTES // max(1, n_samples * elem))
             rows = min(rows, n_chans, 65535)
+            if on_device:
+                self._device_tiles(data, rows, dtype_code, tiles, outlier_boundary)
+                return self._fp32_tiles(tiles, precision)
             in_bytes = rows * n_samples * elem
             slots = self._slots(in_bytes, 16)
             ws_bytes = lib.parrm_channel_scales_workspace_bytes(rows, n_samples)
@@ -258,7 +274,7 @@ class DeviceEngine:
                     _vp(slot["d_in"].data_ptr()), c1 - c0, n_samples, n_samples,
                     _vp(scale.data_ptr() + 8 * c0), _vp(ws_ptr), ws_bytes, dtype_code, run),
                     "parrm_channel_scales")
-                self.launches += 2
+                self._count(2)
                 for tile in tiles:
                     check(lib.parrm_standardise_gather(
                         _vp(slot["d_in"].data_ptr()), c1 - c0, n_samples, n_samples,
@@ -267,20 +283,79 @@ class DeviceEngine:
                         _vp(tile.y.data_ptr() + 8 * c0), n_chans,
                         _vp(tile.sumsq.data_ptr() + 8 * c0), dtype_code, run),
                         "parrm_standardise_gather")
-                    self.launches += 2
+                    self._count(2)
                 slot["ev_run"].record(self.s_run)
                 slot["used"] = True
-            if precision == "fp32":  # float32 storage of the tiles; sums of the rounded values
-                with t.cuda.stream(self.s_run):
-                    for tile in tiles:
-                        tile.y = tile.y.to(t.float32)
-                        check(lib.parrm_channel_sumsq(
-                            _vp(tile.y.data_ptr()), _native.F32, tile.n_chans, tile.n_chans,
-                            tile.n_indices, _vp(tile.sumsq.data_ptr()), run), "parrm_channel_sumsq")
-                        self.launches += 1
             self.s_run.synchronize()
             self._scale = scale
-            return tiles
+            return self._fp32_tiles(tiles, precision)
+
+    def _fp32_tiles(self, tiles, precision):
+        """float32 storage of the tiles in the fp32 mode; channel sums of the rounded values."""
+        t = self.torch
+        if precision == "fp32":
+            with self._lock, t.cuda.device(self.device):
+                sp = self._stream_ptr(t.cuda.current_stream())
+                for tile in tiles:
+                    tile.y = tile.y.to(t.float32)
+                    check(lib.parrm_channel_sumsq(
+                        _vp(tile.y.data_ptr()), _native.F32, tile.n_chans, tile.n_chans,
+                        tile.n_indices, _vp(tile.sumsq.data_ptr()), sp), "parrm_channel_sumsq")
+                    self._count(1)
+                t.cuda.current_stream().synchronize()
+        return tiles
+
+    def _device_recording(self, data):
+        """``(rows-contiguous [C, T] tensor, compute code)`` of a float64 / float32 CUDA recording
+        on this engine's GPU (a row-strided view is copied to a dense tensor first)."""
+        t = self.torch
+        if data.device != self.device:
+            raise ValueError(f"the recording is on {data.device}; this engine runs on {self.device}")
+        code = {t.float64: _native.F64, t.float32: _native.F32}.get(data.dtype)
+        if code is None:
+            raise TypeError(f"unsupported data dtype {data.dtype}")
+        if data.dim() != 2:
+            raise ValueError("`data` must be a 2D array.")
+        if not data.is_contiguous():
+            data = data.contiguous()
+        return data, code
+
+    def _aligned_rows(self, data, c0: int, c1: int):
+        """Channels ``[c0, c1)`` of a dense device recording, based at a 16-byte boundary as the
+        host path's staging slots are (copied when the view's base is not): the scale kernel
+        takes its vector loads, and with them its order of summation, only on aligned rows,
+        so this is what keeps device and host results bit-equal."""
+        block = data[c0:c1]
+        return block if block.data_ptr() % 16 == 0 else block.clone()
+
+    def _device_tiles(self, data, rows, dtype_code, tiles, outlier_boundary):
+        """The device branch of :meth:`prepare_tiles`: the same channel blocks and row stride as
+        the host path's staging slots, read where the recording lies (no H2D)."""
+        t = self.torch
+        n_chans, n_samples = data.shape
+        sp = self._stream_ptr(t.cuda.current_stream())
+        ws_bytes = lib.parrm_channel_scales_workspace_bytes(rows, n_samples)
+        scale = t.empty(n_chans, dtype=t.float64, device=self.device)
+        ws = self._empty(max(ws_bytes, 16), t.uint8)
+        for c0 in range(0, n_chans, rows):
+            c1 = min(c0 + rows, n_chans)
+            block = self._aligned_rows(data, c0, c1)
+            check(lib.parrm_channel_scales(
+                _vp(block.data_ptr()), c1 - c0, n_samples, n_samples,
+                _vp(scale.data_ptr() + 8 * c0), _vp(ws.data_ptr()), ws_bytes, dtype_code, sp),
+                "parrm_channel_scales")
+            self._count(2)
+            for tile in tiles:
+                check(lib.parrm_standardise_gather(
+                    _vp(block.data_ptr()), c1 - c0, n_samples, n_samples,
+                    _vp(tile.indices.data_ptr()), tile.n_indices,
+                    _vp(scale.data_ptr() + 8 * c0), float(outlier_boundary),
+                    _vp(tile.y.data_ptr() + 8 * c0), n_chans,
+                    _vp(tile.sumsq.data_ptr() + 8 * c0), dtype_code, sp),
+                    "parrm_standardise_gather")
+                self._count(2)
+        t.cuda.current_stream().synchronize()
+        self._scale = scale
 
     def tile_from_standardised(self, z: np.ndarray, indices: np.ndarray) -> SearchTile:
         """Tile from an already standardised ``[channels, times]`` host array (the reference's
@@ -295,7 +370,7 @@ class DeviceEngine:
                                           int(y.shape[1]), int(y.shape[0]), _vp(d_sumsq.data_ptr()),
                                           self._stream_ptr(t.cuda.current_stream())),
                   "parrm_channel_sumsq")
-            self.launches += 1
+            self._count(1)
             return SearchTile(
                 y=d_y, sumsq=d_sumsq, indices=t.from_numpy(indices).to(self.device),
                 n_indices=int(y.shape[0]), n_chans=int(y.shape[1]),
@@ -320,19 +395,31 @@ class DeviceEngine:
                               indices=tile.indices, n_indices=tile.n_indices, n_chans=int(n_chans))
 
     def standardise_full(self, data: np.ndarray, outlier_boundary: float) -> np.ndarray:
-        """The reference's ``_standard_data`` array [C, T-1] (parrm.py:272-280), on demand."""
+        """The reference's ``_standard_data`` array [C, T-1] (parrm.py:272-280), on demand; a
+        CUDA tensor for a CUDA recording."""
         t = self.torch
-        data, dtype_code = self._as_float_array(data, allow_f32=True)
-        n_chans, n_samples = data.shape
-        out = np.empty((n_chans, n_samples - 1), dtype=data.dtype)
+        on_device = not isinstance(data, np.ndarray)
+        if on_device:  # a CUDA recording: read where it lies, a device tensor comes back
+            data, dtype_code = self._device_recording(data)
+            n_chans, n_samples = data.shape
+            out = t.empty((n_chans, n_samples - 1), dtype=data.dtype, device=self.device)
+            elem = data.element_size()
+        else:
+            data, dtype_code = self._as_float_array(data, allow_f32=True)
+            n_chans, n_samples = data.shape
+            out = np.empty((n_chans, n_samples - 1), dtype=data.dtype)
+            elem = data.dtype.itemsize
         tdtype = t.float64 if dtype_code == _native.F64 else t.float32
-        rows = max(1, min(n_chans, 65535, _CHUNK_BYTES // max(1, n_samples * data.dtype.itemsize)))
+        rows = max(1, min(n_chans, 65535, _CHUNK_BYTES // max(1, n_samples * elem)))
         with self._lock, t.cuda.device(self.device):
             stream = t.cuda.current_stream()
             sp = self._stream_ptr(stream)
             for c0 in range(0, n_chans, rows):
                 c1 = min(c0 + rows, n_chans)
-                d_x = t.from_numpy(np.ascontiguousarray(data[c0:c1])).to(self.device)
+                if on_device:
+                    d_x = self._aligned_rows(data, c0, c1)
+                else:
+                    d_x = t.from_numpy(np.ascontiguousarray(data[c0:c1])).to(self.device)
                 scale = t.empty(c1 - c0, dtype=t.float64, device=self.device)
                 ws_bytes = lib.parrm_channel_scales_workspace_bytes(c1 - c0, n_samples)
                 ws = self._empty(max(ws_bytes, 16), t.uint8)
@@ -345,8 +432,8 @@ class DeviceEngine:
                                                  float(outlier_boundary), _vp(d_z.data_ptr()),
                                                  n_samples - 1, dtype_code, sp),
                       "parrm_standardise_full")
-                self.launches += 3
-                out[c0:c1] = d_z.cpu().numpy()
+                self._count(3)
+                out[c0:c1] = d_z if on_device else d_z.cpu().numpy()
         return out
 
     def evaluate(
@@ -398,8 +485,8 @@ class DeviceEngine:
                                                             bandwidth, code)
                 if self._eval_ws.numel() < need:
                     self._eval_ws = self._empty(need, t.uint8)
-                self.launches += self._eval_into(tile, d_per[p0:p1], d_err[p0:p1], bandwidth,
-                                                 lambda_, n_chans_divisor, sp)
+                self._count(self._eval_into(tile, d_per[p0:p1], d_err[p0:p1], bandwidth,
+                                            lambda_, n_chans_divisor, sp))
             return d_err
 
     def _eval_into(self, tile, d_per, d_err, bandwidth, lambda_, n_chans_divisor, sp) -> int:
@@ -463,7 +550,7 @@ class DeviceEngine:
             check(lib.parrm_nm_init(_vp(d_starts.data_ptr()), n, _vp(d_state.data_ptr()),
                                     _vp(d_points.data_ptr()), sp), "parrm_nm_init")
             one_round(sp)  # the initial simplex; also loads every kernel before the capture
-            self.launches += 1 + kernels_per_round[0]
+            self._count(1 + kernels_per_round[0])
             active = int(d_active.item())
             if active:
                 # capture_begin / capture_end directly: torch.cuda.graph() also runs
@@ -483,8 +570,8 @@ class DeviceEngine:
                     graph.replay()
                     replays += 1
                     active = int(d_active.item())
-                self.launches += replays            # one launch per replay ...
-                self.graph_kernels += replays * self.ROUNDS_PER_GRAPH * kernels_per_round[0]
+                self._count(replays,            # one launch per replay ...
+                            graph_kernels=replays * self.ROUNDS_PER_GRAPH * kernels_per_round[0])
             raw = d_state.cpu().numpy().view(np.dtype([
                 ("sim", np.float64, 2), ("fsim", np.float64, 2), ("points", np.float64, 5),
                 ("fcalls", np.int32), ("iterations", np.int32), ("done", np.int32),
@@ -501,7 +588,7 @@ class DeviceEngine:
             check(lib.parrm_argmin(_vp(d_values.data_ptr()), int(d_values.shape[0]),
                                    _vp(d_val.data_ptr()), _vp(d_idx.data_ptr()),
                                    self._stream_ptr(t.cuda.current_stream())), "parrm_argmin")
-            self.launches += 1
+            self._count(1)
             return float(d_val.item()), int(d_idx.item())
 
     # --------------------------------------------------------------------- taps
@@ -519,7 +606,7 @@ class DeviceEngine:
                 int(omit_n_samples), _native.DIRECTIONS[direction], _vp(d_taps.data_ptr()),
                 _vp(d_n.data_ptr()), self._stream_ptr(t.cuda.current_stream())),
                 "parrm_build_taps")
-            self.launches += 1
+            self._count(1)
             n = int(d_n.item())
             return d_taps[:n].cpu().numpy()
 
@@ -538,7 +625,7 @@ class DeviceEngine:
                 _vp(d_per.data_ptr()), _vp(d_phw.data_ptr()), _vp(d_omit.data_ptr()),
                 _vp(d_lim.data_ptr()), n, _vp(d_out.data_ptr()),
                 self._stream_ptr(t.cuda.current_stream())), "parrm_default_half_width")
-            self.launches += 1
+            self._count(1)
             return d_out.cpu().numpy()
 
     def filter_sweep(self, data: np.ndarray, periods, period_half_widths, half_widths, omits,
@@ -572,7 +659,7 @@ class DeviceEngine:
                 _vp(d_x.data_ptr()), n_samples, n_samples, n_chans, _vp(d_taps.data_ptr()), stride,
                 _vp(d_n.data_ptr()), n_sets, max_hw, _vp(d_out.data_ptr()), n_samples,
                 n_chans * n_samples, code, sp), "parrm_filter_apply_batch")
-            self.launches += 2
+            self._count(2)
             self.last_filter_kernel = _native.filter_last_kernel()
             counts = d_n.cpu().numpy()
             taps_all = d_taps.cpu().numpy()
@@ -606,7 +693,7 @@ class DeviceEngine:
                     _vp(d_x[c0:c1].data_ptr()), c1 - c0, n_samples, d_x.stride(0), code,
                     int(n_points), float(sampling_freq), _vp(d_psd[c0:c1].data_ptr()), n_bins,
                     self._stream_ptr(t.cuda.current_stream())), "parrm_periodogram")
-                self.launches += 1
+                self._count(1)
             psd = d_psd.cpu().numpy()
         return psd[0] if one_d else psd
 
@@ -726,7 +813,7 @@ class DeviceEngine:
                 opts, _vp(d_x[c0:c1].data_ptr()), d_x.stride(0), 0, n_samples,
                 _vp(d_out[c0:c1].data_ptr()), d_out.stride(0), 0, n_samples, n_samples, c1 - c0,
                 _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), code, self._stream_ptr(stream))
-            self.launches += 1
+            self._count(1)
         return d_out
 
     def filter_shard(self, chunk: np.ndarray, taps: np.ndarray, x0: int, t0: int, t1: int,
@@ -754,7 +841,7 @@ class DeviceEngine:
                     opts, _vp(d_x[c0:c1].data_ptr()), n_x, x0, n_x, _vp(d_out[c0:c1].data_ptr()),
                     t1 - t0, t0, t1 - t0, n_total, c1 - c0, _vp(d_plan.data_ptr()),
                     _vp(h_plan.ctypes.data), code, self._stream_ptr(t.cuda.current_stream()))
-                self.launches += 1
+                self._count(1)
             return d_out.to(t.float64)
 
     def filter_host_window(self, chunk: np.ndarray, taps: np.ndarray, x0: int, t0: int, t1: int,
@@ -845,17 +932,17 @@ class DeviceEngine:
                 if widen_in:
                     check(lib.parrm_convert(_vp(d_x), in_code, _vp(slot["d_x"].data_ptr()),
                                             comp_code, n_c * n_x, s_run), "parrm_convert")
-                    self.launches += 1
+                    self._count(1)
                     d_x = slot["d_x"].data_ptr()
                 d_y = slot["d_y"].data_ptr() if narrow_out else slot["d_out"].data_ptr()
                 self._apply(
                     opts, _vp(d_x), n_x, x0, n_x, _vp(d_y), n_o, t0, n_o, n_samples,
                     n_c, _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), comp_code, s_run)
-                self.launches += 1
+                self._count(1)
                 if narrow_out:
                     check(lib.parrm_convert(_vp(d_y), comp_code, _vp(slot["d_out"].data_ptr()),
                                             out_code, n_c * n_o, s_run), "parrm_convert")
-                    self.launches += 1
+                    self._count(1)
                 slot["ev_run"].record(self.s_run)
                 self.s_out.wait_event(slot["ev_run"])
                 if out_pinned:
@@ -874,33 +961,68 @@ class DeviceEngine:
         return out
 
     # ------------------------------------------------------------- streaming
-    _STREAM_HEADER = 64      # bytes before the block in the staging buffers: the position
+    # A stream's pushes take the stream's own lock, never the engine's ``_lock``: a period
+    # search in another host thread (which holds ``_lock`` for each of its steps) must not
+    # stall the acquisition loop.  They touch no shared engine state but the counters
+    # (``_count``); ``parrm_host_copy`` serialises its callers itself.
+    _STREAM_HEADER = 64      # bytes before the block in the staging buffers: {pos, out_lo}
     _STREAM_GRAPHS = 4       # captured push shapes kept per stream
 
-    def stream_open(self, taps: np.ndarray, max_chunk: int, precision: str = "fp64"):
+    def stream_open(self, taps: np.ndarray, max_chunk: int, precision: str = "fp64",
+                    history: int = 0):
         """State of one streaming filter (:mod:`pyparrm_b200._stream`): taps on the device, a
         CUDA stream of its own, and -- from the first push, which fixes the channel count -- the
-        ring of the last ``span + max_chunk`` samples per channel and pinned in/out staging.
-        Two streams never share any of it."""
+        ring of the last ``max(span, history) + max_chunk`` samples per channel and pinned
+        in/out staging.  Two streams never share any of it."""
         t = self.torch
         taps = np.ascontiguousarray(taps, dtype=np.int32)
-        with self._lock, t.cuda.device(self.device):
+        span = max(int(taps[-1]), 0) - min(int(taps[0]), 0)
+        with t.cuda.device(self.device):
             return _StreamState(
                 taps=taps, d_taps=t.from_numpy(taps).to(self.device), max_chunk=int(max_chunk),
                 code=_native.F32 if precision == "fp32" else _native.F64,
                 latency=max(0, -int(taps[0])), device=self.device,
-                stream=t.cuda.Stream(device=self.device))
+                stream=t.cuda.Stream(device=self.device),
+                ring_len=max(span, int(history)) + int(max_chunk))
+
+    def stream_retune(self, st, taps: np.ndarray) -> None:
+        """Switch an open stream to new taps (``FilterStream.set_filter``, which has checked
+        that the ring holds what they read).  The upload runs on the stream's CUDA stream,
+        after its pushes so far; the old tap tensor is kept until those have finished."""
+        t = self.torch
+        taps = np.ascontiguousarray(taps, dtype=np.int32)
+        with st.lock, t.cuda.device(self.device):
+            with t.cuda.stream(st.stream):
+                d_taps = t.from_numpy(taps).to(self.device)
+            st.d_taps.record_stream(st.stream)
+            st.taps, st.d_taps, st.latency = taps, d_taps, max(0, -int(taps[0]))
+            st.graphs.clear()
+            st.seen.clear()
+
+    def stream_recent(self, st, n: int, pos: int):
+        """The last ``n`` of the ``pos`` samples pushed, ``[channels, n]`` in the compute type,
+        copied out of the ring on the stream's CUDA stream (after its pushes); the caller's
+        current stream waits for the copy."""
+        t = self.torch
+        with st.lock, t.cuda.device(self.device):
+            comp = t.float32 if st.code == _native.F32 else t.float64
+            out = t.empty((st.n_chans, int(n)), dtype=comp, device=self.device)
+            current = t.cuda.current_stream()
+            st.stream.wait_stream(current)
+            check(lib.parrm_stream_window(
+                _vp(st.ring.data_ptr()), st.ring_len, st.n_chans, int(pos), int(n),
+                _vp(out.data_ptr()), int(n), st.code, self._stream_ptr(st.stream)),
+                "parrm_stream_window")
+            current.wait_stream(st.stream)
+            return out
 
     def _stream_buffers(self, st, n_chans: int, in_bytes: int, out_bytes: int) -> None:
         """Ring at the first push; staging grown to the largest push (captured graphs hold the
         old pointers, so growing drops them)."""
         t = self.torch
         if st.ring is None:
-            nbytes = lib.parrm_stream_ring_bytes(n_chans, _vp(st.taps.ctypes.data),
-                                                 int(st.taps.shape[0]), st.max_chunk, st.code)
-            if nbytes == 0:
-                check(1, "parrm_stream_ring_bytes")
-            st.ring = self._empty(nbytes, t.uint8)
+            st.ring = self._empty(n_chans * st.ring_len * (4 if st.code == _native.F32 else 8),
+                                  t.uint8)
             st.n_chans = n_chans
         in_bytes += self._STREAM_HEADER
         if st.d_in is None or st.d_in.numel() < in_bytes:
@@ -913,36 +1035,38 @@ class DeviceEngine:
             st.graphs.clear()
 
     def _stream_launch(self, st, d_block, block_code, ld_block, n, d_out, out_code, k, pos,
-                       d_pos, close, sp) -> None:
+                       out_lo, d_hdr, close, sp) -> None:
         w_min, w_max = int(st.taps[0]), int(st.taps[-1])
-        check(lib.parrm_stream_push(
-            _vp(st.ring.data_ptr()), st.n_chans, st.max_chunk, _vp(st.d_taps.data_ptr()),
+        check(lib.parrm_stream_push_at(
+            _vp(st.ring.data_ptr()), st.ring_len, st.n_chans, _vp(st.d_taps.data_ptr()),
             int(st.taps.shape[0]), w_min, w_max, _vp(d_block), block_code, ld_block, n,
-            _vp(d_out), out_code, max(k, 1), pos, d_pos, int(close), st.code, sp),
-            "parrm_stream_push")
+            _vp(d_out), out_code, max(k, 1), pos, out_lo, d_hdr, int(close), st.code, sp),
+            "parrm_stream_push_at")
 
-    def stream_push(self, st, block, pos: int, close: bool, out_dtype=None, graphs: bool = False):
+    def stream_push(self, st, block, pos: int, close: bool, out_dtype=None, graphs: bool = False,
+                    emitted: int | None = None):
         """One push (``block`` None: nothing new, the closing push): returns the outputs it makes
-        final, ``_stream.output_range``.  NumPy blocks go through the stream's pinned staging
+        final, ``_stream.output_range`` (from ``emitted``, the outputs returned so far, once the
+        stream's taps have been switched).  NumPy blocks go through the stream's pinned staging
         (H2D, one kernel, D2H, on the stream's own CUDA stream); with ``graphs``, a push of the
-        same shape as an earlier one, on an open stream past its latency, is captured once and
-        then replayed as one CUDA graph that reads the position from a header copied up with
-        the block.  CUDA blocks are read where they lie and a CUDA tensor comes back."""
+        same shape as an earlier one that returns exactly one output per sample is captured
+        once and then replayed as one CUDA graph that reads the positions from a header copied
+        up with the block.  CUDA blocks are read where they lie and a CUDA tensor comes back."""
         from ._stream import output_range
 
         t = self.torch
-        with self._lock, t.cuda.device(self.device):
+        with st.lock, t.cuda.device(self.device):
             if st.on_device is None:
                 st.on_device = block is not None and not isinstance(block, np.ndarray)
             if st.on_device:
-                return self._stream_push_device(st, block, pos, close, output_range)
+                return self._stream_push_device(st, block, pos, close, emitted, output_range)
             if block is None:
                 block = np.zeros((st.n_chans, 0), dtype=np.float64)
             data, in_code = self._as_storage_array(block)
             n_chans, n = data.shape
             out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
             out_code = _native.F64 if out_np == np.float64 else _native.F32
-            lo, hi = output_range(pos, n, st.latency, close)
+            lo, hi = output_range(pos, n, st.latency, close, emitted)
             k = hi - lo
             in_bytes, out_bytes = data.nbytes, n_chans * k * out_np.itemsize
             self._stream_buffers(st, n_chans, in_bytes, out_bytes)
@@ -953,22 +1077,22 @@ class DeviceEngine:
                 _threaded_memmove(h_in + hdr, data.ctypes.data, in_bytes)
             sp = self._stream_ptr(st.stream)
             key = (n_chans, n, in_code, out_code)
-            replayable = graphs and not close and pos >= st.latency and n > 0
+            replayable = graphs and not close and k == n and n > 0
             if replayable and (key in st.graphs or key in st.seen):
-                st.stage_in[:8].numpy().view(np.int64)[0] = pos
+                st.stage_in[:16].numpy().view(np.int64)[:] = (pos, lo)
                 graph = st.graphs.get(key)
                 if graph is None:
-                    graph = self._stream_capture(st, key, data.shape, in_code, out_code, k, pos)
+                    graph = self._stream_capture(st, key, data.shape, in_code, out_code, k, pos,
+                                                 lo)
                 with t.cuda.stream(st.stream):
                     graph.replay()
-                self.launches += 1
-                self.graph_kernels += 1
+                self._count(1, graph_kernels=1)
             else:
                 check(lib.parrm_copy_h2d_async(_vp(d_in + hdr), _vp(h_in + hdr), in_bytes, sp),
                       "H2D copy")
-                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos, None,
-                                    close, sp)
-                self.launches += 1
+                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos, lo,
+                                    None, close, sp)
+                self._count(1)
                 check(lib.parrm_copy_d2h_async(_vp(h_out), _vp(d_out), out_bytes, sp), "D2H copy")
                 if replayable:
                     st.seen.add(key)
@@ -976,7 +1100,7 @@ class DeviceEngine:
             view = st.stage_out[:out_bytes].numpy().view(out_np).reshape(n_chans, k)
             return view.copy()
 
-    def _stream_capture(self, st, key, shape, in_code, out_code, k, pos):
+    def _stream_capture(self, st, key, shape, in_code, out_code, k, pos, lo):
         """Capture H2D (header + block) -> kernel -> D2H of a push shape as one CUDA graph."""
         t = self.torch
         n_chans, n = shape
@@ -992,7 +1116,7 @@ class DeviceEngine:
             try:
                 check(lib.parrm_copy_h2d_async(_vp(d_in), _vp(h_in), hdr + n_chans * n * es_in, sp),
                       "H2D copy")
-                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos,
+                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos, lo,
                                     _vp(d_in), False, sp)
                 check(lib.parrm_copy_d2h_async(_vp(h_out), _vp(d_out), n_chans * k * es_out, sp),
                       "D2H copy")
@@ -1006,7 +1130,7 @@ class DeviceEngine:
     _TORCH_STORAGE = {"torch.float64": _native.F64, "torch.float32": _native.F32,
                       "torch.int16": _native.I16, "torch.int32": _native.I32}
 
-    def _stream_push_device(self, st, block, pos, close, output_range):
+    def _stream_push_device(self, st, block, pos, close, emitted, output_range):
         t = self.torch
         comp = t.float32 if st.code == _native.F32 else t.float64
         if block is None:
@@ -1017,14 +1141,14 @@ class DeviceEngine:
         if block.stride(1) != 1 and block.shape[1] > 1:
             block = block.contiguous()
         n_chans, n = block.shape
-        lo, hi = output_range(pos, n, st.latency, close)
+        lo, hi = output_range(pos, n, st.latency, close, emitted)
         self._stream_buffers(st, n_chans, 0, 0)
         out = t.empty((n_chans, hi - lo), dtype=comp, device=self.device)
         current = t.cuda.current_stream()
         st.stream.wait_stream(current)
         self._stream_launch(st, block.data_ptr(), code, max(block.stride(0), n), n, out.data_ptr(),
-                            st.code, hi - lo, pos, None, close, self._stream_ptr(st.stream))
-        self.launches += 1
+                            st.code, hi - lo, pos, lo, None, close, self._stream_ptr(st.stream))
+        self._count(1)
         current.wait_stream(st.stream)
         return out
 

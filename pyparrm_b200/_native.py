@@ -20,7 +20,7 @@ DIR_BOTH, DIR_PAST, DIR_FUTURE = 0, 1, 2
 DIRECTIONS = {"both": DIR_BOTH, "past": DIR_PAST, "future": DIR_FUTURE}
 MAX_BANDWIDTH = 23
 NM_STATE_BYTES = 88
-ABI_VERSION = 7
+ABI_VERSION = 8
 PLAN_AUTO, PLAN_GATHER, PLAN_COMB = 0, 1, 2
 KERNEL_AUTO, KERNEL_GATHER, KERNEL_SPECIALISED = 0, 1, 3
 
@@ -129,6 +129,14 @@ SIGNATURES = {
         [c_void_p, c_int64, c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int,
          c_int64, c_int64, c_void_p, c_int, c_int64, c_int64, c_void_p, c_int, c_int, c_void_p],
     ),
+    "parrm_stream_push_at": (
+        c_int,
+        [c_void_p, c_int64, c_int64, c_void_p, c_int32, c_int32, c_int32, c_void_p, c_int,
+         c_int64, c_int64, c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int,
+         c_void_p],
+    ),
+    "parrm_stream_window": (
+        c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int, c_void_p]),
     "parrm_fp64_fma_burn": (c_int, [c_int64, c_void_p, POINTER(c_double), c_void_p]),
 }
 

@@ -4,20 +4,25 @@
 //   ring[c * R + (t mod R)]  the last R samples of every channel, in the compute type, with
 //                            R = span + max_chunk,  span = max(w_max, 0) - min(w_min, 0);
 //   taps                     ascending offsets, as parrm_build_taps produces them;
-//   pos                      samples pushed before this block (a host argument, or a device
-//                            int64 so that a captured CUDA graph can replay with a new position).
+//   pos, out_lo              samples pushed before this block and the first output not yet
+//                            written (host arguments, or a device int64 header so that a
+//                            captured CUDA graph can replay with new positions).
 //
 // One launch per push.  The block holds samples [pos, pos + n) in its storage type.  Output t
 // reads samples t - w for the taps w; it is final once sample t + L exists, L = max(0, -w_min),
-// so while the stream is open a push produces outputs [max(0, pos - L), pos + n - L) and the
+// so while the stream is open a push produces outputs [out_lo, max(out_lo, pos + n - L)) and the
 // closing push the rest, up to pos + n, with the recording-end edge.  Treating the recording as
-// ending at pos + n is exact for the open outputs too: none of their taps reaches past it.
+// ending at pos + n is exact for the open outputs too: none of their taps reaches past it.  With
+// one tap set for the whole stream out_lo = max(0, pos - L) (parrm_stream_push); after a switch
+// of taps the caller passes it (parrm_stream_push_at), and a push can then emit more or fewer
+// than n outputs.
 //
 // Every CTA reads samples >= pos from the incoming block and older ones from the ring, and
 // writes only its own slice of the block into the ring.  The oldest sample any output of this
-// launch reads is pos - span, and R >= span + n, so the slots written here ((pos .. pos+n-1)
-// mod R) are never slots read here: no grid-wide barrier is needed.  Work and traffic per push
-// are O(channels x (n + span)), independent of how much has been pushed.
+// launch reads is out_lo - w_max, and the caller guarantees R >= pos + n - that (R >= span + n
+// for a single tap set), so the slots written here ((pos .. pos+n-1) mod R) are never slots read
+// here: no grid-wide barrier is needed.  Work and traffic per push are O(channels x (n + span +
+// pos - out_lo)), independent of how much has been pushed.
 //
 // Arithmetic: the same floating-point operations in the same order as the gather kernels of
 // filter.cu (ascending taps, sequential adds, acc / n_taps in the interior, acc / n_in at the
@@ -42,10 +47,10 @@ struct StreamArgs {
   const int32_t* taps;
   const void* block;
   void* out;
-  const int64_t* d_pos;
-  int64_t ring_len, ld_block, n, ld_out, pos;
+  const int64_t* d_hdr;  // {pos} (hdr_words 1) or {pos, out_lo} (hdr_words 2), or NULL
+  int64_t ring_len, ld_block, n, ld_out, pos, out_lo;
   int32_t n_taps, w_lo, w_hi, tile;
-  int32_t block_type, out_type, close;
+  int32_t block_type, out_type, close, hdr_words;
 };
 
 template <typename T>
@@ -79,9 +84,14 @@ struct StreamRange {
 template <typename T>
 __device__ __forceinline__ StreamRange stream_range(const StreamArgs<T>& a) {
   StreamRange r;
-  r.pos = a.d_pos ? *a.d_pos : a.pos;
   const int64_t lat = -int64_t(a.w_lo);
-  r.out_lo = max(int64_t(0), r.pos - lat);
+  if (a.d_hdr == nullptr) {
+    r.pos = a.pos;
+    r.out_lo = a.out_lo;
+  } else {
+    r.pos = a.d_hdr[0];
+    r.out_lo = a.hdr_words == 2 ? a.d_hdr[1] : max(int64_t(0), r.pos - lat);
+  }
   r.n_total = r.pos + a.n;
   r.out_hi = a.close ? r.n_total : max(r.out_lo, r.n_total - lat);
   return r;
@@ -124,7 +134,7 @@ stream_gather_smem_kernel(const StreamArgs<T> a) {
   const int64_t v_mid = max(v_lo, min(g_hi, r.pos));  // [v_lo, v_mid) from the ring
   const int64_t v_hi = min(g_hi, r.n_total);          // [v_mid, v_hi) from the block
   const T* ring = a.ring + chan * a.ring_len;
-  const int64_t ring0 = v_lo % a.ring_len;            // at most span samples: one wrap at most
+  const int64_t ring0 = v_lo % a.ring_len;            // fewer than R samples: one wrap at most
 
   for (int i = tid; i < a.n_taps; i += kStreamThreads) s_taps[i] = a.taps[i];
   for (int i = tid; i < int(g_hi - g_lo); i += kStreamThreads) {
@@ -221,6 +231,7 @@ static int64_t stream_span(int32_t w_min, int32_t w_max) {
 
 template <typename T>
 int launch_stream(StreamArgs<T> a, int64_t n_chans, int64_t n_out_max, cudaStream_t stream) {
+  // n_out_max covers both the outputs and the block: CTA x also writes block slice x to the ring
   const int64_t span = int64_t(a.w_hi) - a.w_lo;
   const int64_t fixed = round16s(a.n_taps * 4);
   const int64_t es = int64_t(sizeof(T));
@@ -271,6 +282,47 @@ size_t parrm_stream_ring_bytes(int64_t n_chans, const int32_t* h_taps, int32_t n
   return size_t(n_chans) * size_t(ring_len) * (dtype == PARRM_F64 ? 8 : 4);
 }
 
+// The body of both push entry points: arguments already checked except those below.
+static int stream_push_impl(const char* fn, void* d_ring, int64_t ring_len, int64_t n_chans,
+                            const int32_t* d_taps, int32_t n_taps, int32_t w_min, int32_t w_max,
+                            const void* d_block, int block_type, int64_t ld_block, int64_t n,
+                            void* d_out, int out_type, int64_t ld_out, int64_t pos,
+                            int64_t out_lo, int64_t n_grid, const int64_t* d_hdr, int hdr_words,
+                            int close, int dtype, void* stream) {
+  using namespace parrm;
+  PARRM_REQUIRE(dtype == PARRM_F64 || dtype == PARRM_F32, "%s: bad dtype %d", fn, dtype);
+  PARRM_REQUIRE(out_type == PARRM_F64 || out_type == PARRM_F32, "%s: bad output type %d", fn,
+                out_type);
+  PARRM_REQUIRE(block_type == PARRM_F64 || block_type == PARRM_F32 || block_type == PARRM_I16 ||
+                    block_type == PARRM_I32,
+                "%s: unknown block storage type %d", fn, block_type);
+  PARRM_REQUIRE(n_chans >= 1 && n_chans <= 65535, "%s: 1..65535 channels, got %lld", fn,
+                (long long)n_chans);
+  PARRM_REQUIRE(n_taps >= 1 && w_min <= w_max, "%s: empty or unordered tap list", fn);
+  PARRM_REQUIRE(d_ring != nullptr && d_taps != nullptr, "%s: null ring or taps", fn);
+  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
+  const int64_t out_hi = close ? pos + n : (pos + n - lat > out_lo ? pos + n - lat : out_lo);
+  if (n == 0 && out_hi == out_lo) return PARRM_OK;
+  PARRM_REQUIRE(n == 0 || (d_block != nullptr && ld_block >= n),
+                "%s: null block or row stride %lld < %lld", fn, (long long)ld_block,
+                (long long)n);
+  PARRM_REQUIRE(out_hi == out_lo || (d_out != nullptr && ld_out >= out_hi - out_lo),
+                "%s: null output or row stride %lld < %lld outputs", fn, (long long)ld_out,
+                (long long)(out_hi - out_lo));
+  const int32_t w_lo = w_min < 0 ? w_min : 0, w_hi = w_max > 0 ? w_max : 0;
+  cudaStream_t s = as_stream(stream);
+  if (dtype == PARRM_F64) {
+    StreamArgs<double> a{static_cast<double*>(d_ring), d_taps, d_block, d_out, d_hdr, ring_len,
+                         ld_block, n, ld_out, pos, out_lo, n_taps, w_lo, w_hi, 0, block_type,
+                         out_type, close ? 1 : 0, hdr_words};
+    return launch_stream<double>(a, n_chans, n_grid, s);
+  }
+  StreamArgs<float> a{static_cast<float*>(d_ring), d_taps, d_block, d_out, d_hdr, ring_len,
+                      ld_block, n, ld_out, pos, out_lo, n_taps, w_lo, w_hi, 0, block_type,
+                      out_type, close ? 1 : 0, hdr_words};
+  return launch_stream<float>(a, n_chans, n_grid, s);
+}
+
 int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const int32_t* d_taps,
                       int32_t n_taps, int32_t w_min, int32_t w_max, const void* d_block,
                       int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
@@ -278,15 +330,6 @@ int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const in
                       void* stream) {
   PARRM_NVTX("parrm_stream_push");
   using namespace parrm;
-  PARRM_REQUIRE(dtype == PARRM_F64 || dtype == PARRM_F32, "parrm_stream_push: bad dtype %d", dtype);
-  PARRM_REQUIRE(out_type == PARRM_F64 || out_type == PARRM_F32,
-                "parrm_stream_push: bad output type %d", out_type);
-  PARRM_REQUIRE(block_type == PARRM_F64 || block_type == PARRM_F32 || block_type == PARRM_I16 ||
-                    block_type == PARRM_I32,
-                "parrm_stream_push: unknown block storage type %d", block_type);
-  PARRM_REQUIRE(n_chans >= 1 && n_chans <= 65535, "parrm_stream_push: 1..65535 channels, got %lld",
-                (long long)n_chans);
-  PARRM_REQUIRE(n_taps >= 1 && w_min <= w_max, "parrm_stream_push: empty or unordered tap list");
   PARRM_REQUIRE(max_chunk >= 1, "parrm_stream_push: max_chunk must be >= 1");
   PARRM_REQUIRE(n >= 0 && n <= max_chunk,
                 "parrm_stream_push: block of %lld samples is longer than the ring allows "
@@ -295,31 +338,78 @@ int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const in
                 (long long)pos);
   PARRM_REQUIRE(pos <= INT64_MAX / 2, "parrm_stream_push: position %lld out of range",
                 (long long)pos);
-  PARRM_REQUIRE(d_ring != nullptr && d_taps != nullptr, "parrm_stream_push: null ring or taps");
+  // one tap set for the whole stream: the ring of parrm_stream_ring_bytes and the first output
+  // that follows from the position
   const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
   const int64_t out_lo = pos - lat > 0 ? pos - lat : 0;
+  const int64_t n_grid = n + (close ? lat : 0);  // grid extent; independent of pos
+  return stream_push_impl("parrm_stream_push", d_ring, stream_span(w_min, w_max) + max_chunk,
+                          n_chans, d_taps, n_taps, w_min, w_max, d_block, block_type, ld_block,
+                          n, d_out, out_type, ld_out, pos, out_lo, n_grid, d_pos, 1, close, dtype,
+                          stream);
+}
+
+int parrm_stream_push_at(void* d_ring, int64_t ring_len, int64_t n_chans, const int32_t* d_taps,
+                         int32_t n_taps, int32_t w_min, int32_t w_max, const void* d_block,
+                         int block_type, int64_t ld_block, int64_t n, void* d_out, int out_type,
+                         int64_t ld_out, int64_t pos, int64_t out_lo, const int64_t* d_hdr,
+                         int close, int dtype, void* stream) {
+  PARRM_NVTX("parrm_stream_push_at");
+  using namespace parrm;
+  const char* fn = "parrm_stream_push_at";
+  PARRM_REQUIRE(n >= 0, "%s: negative block length %lld", fn, (long long)n);
+  PARRM_REQUIRE(pos >= 0 && pos <= INT64_MAX / 2, "%s: position %lld out of range", fn,
+                (long long)pos);
+  PARRM_REQUIRE(out_lo >= 0 && out_lo <= pos,
+                "%s: first output %lld outside [0, pos = %lld]", fn, (long long)out_lo,
+                (long long)pos);
+  PARRM_REQUIRE(n_taps >= 1 && w_min <= w_max, "%s: empty or unordered tap list", fn);
+  PARRM_REQUIRE(ring_len >= 1, "%s: ring length %lld must be >= 1", fn, (long long)ring_len);
+  // every sample this launch reads, [max(0, out_lo - w_max), pos + n), spans at most the ring:
+  // all of it is still there and no slot written here is read here
+  const int64_t oldest = out_lo - (w_max > 0 ? w_max : 0);
+  const int64_t reach = pos + n - (oldest > 0 ? oldest : 0);
+  PARRM_REQUIRE(reach <= ring_len,
+                "%s: the push reads %lld samples back from pos + n, more than the ring of %lld "
+                "holds (a shorter block, or a longer ring)", fn, (long long)reach,
+                (long long)ring_len);
+  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
   const int64_t out_hi = close ? pos + n : (pos + n - lat > out_lo ? pos + n - lat : out_lo);
-  const int64_t n_out_max = n + (close ? lat : 0);  // grid extent; independent of pos
-  if (n == 0 && out_hi == out_lo) return PARRM_OK;
-  PARRM_REQUIRE(n == 0 || (d_block != nullptr && ld_block >= n),
-                "parrm_stream_push: null block or row stride %lld < %lld", (long long)ld_block,
+  const int64_t n_grid = n > out_hi - out_lo ? n : out_hi - out_lo;
+  return stream_push_impl(fn, d_ring, ring_len, n_chans, d_taps, n_taps, w_min, w_max, d_block,
+                          block_type, ld_block, n, d_out, out_type, ld_out, pos, out_lo, n_grid,
+                          d_hdr, 2, close, dtype, stream);
+}
+
+int parrm_stream_window(const void* d_ring, int64_t ring_len, int64_t n_chans, int64_t pos,
+                        int64_t n, void* d_dst, int64_t ld_dst, int dtype, void* stream) {
+  PARRM_NVTX("parrm_stream_window");
+  using namespace parrm;
+  const char* fn = "parrm_stream_window";
+  PARRM_REQUIRE(dtype == PARRM_F64 || dtype == PARRM_F32, "%s: bad dtype %d", fn, dtype);
+  PARRM_REQUIRE(n_chans >= 1, "%s: need channels >= 1, got %lld", fn, (long long)n_chans);
+  PARRM_REQUIRE(ring_len >= 1, "%s: ring length %lld must be >= 1", fn, (long long)ring_len);
+  PARRM_REQUIRE(n >= 1 && n <= pos && n <= ring_len,
+                "%s: window of %lld samples outside [1, min(pos = %lld, ring = %lld)]", fn,
+                (long long)n, (long long)pos, (long long)ring_len);
+  PARRM_REQUIRE(d_ring != nullptr && d_dst != nullptr && ld_dst >= n,
+                "%s: null ring or destination, or row stride %lld < %lld", fn, (long long)ld_dst,
                 (long long)n);
-  PARRM_REQUIRE(out_hi == out_lo || (d_out != nullptr && ld_out >= out_hi - out_lo),
-                "parrm_stream_push: null output or row stride %lld < %lld outputs",
-                (long long)ld_out, (long long)(out_hi - out_lo));
-  const int64_t ring_len = stream_span(w_min, w_max) + max_chunk;
-  const int32_t w_lo = w_min < 0 ? w_min : 0, w_hi = w_max > 0 ? w_max : 0;
+  // samples [pos - n, pos) sit in slots [first, first + n) mod R: two column ranges at most
+  const size_t es = dtype == PARRM_F64 ? 8 : 4;
+  const int64_t first = (pos - n) % ring_len;
+  const int64_t n1 = n < ring_len - first ? n : ring_len - first;
   cudaStream_t s = as_stream(stream);
-  if (dtype == PARRM_F64) {
-    StreamArgs<double> a{static_cast<double*>(d_ring), d_taps, d_block, d_out, d_pos, ring_len,
-                         ld_block, n, ld_out, pos, n_taps, w_lo, w_hi, 0, block_type, out_type,
-                         close ? 1 : 0};
-    return launch_stream<double>(a, n_chans, n_out_max, s);
-  }
-  StreamArgs<float> a{static_cast<float*>(d_ring), d_taps, d_block, d_out, d_pos, ring_len,
-                      ld_block, n, ld_out, pos, n_taps, w_lo, w_hi, 0, block_type, out_type,
-                      close ? 1 : 0};
-  return launch_stream<float>(a, n_chans, n_out_max, s);
+  const char* ring = static_cast<const char*>(d_ring);
+  char* dst = static_cast<char*>(d_dst);
+  PARRM_CUDA_OK(cudaMemcpy2DAsync(dst, size_t(ld_dst) * es, ring + size_t(first) * es,
+                                  size_t(ring_len) * es, size_t(n1) * es, size_t(n_chans),
+                                  cudaMemcpyDeviceToDevice, s));
+  if (n1 < n)
+    PARRM_CUDA_OK(cudaMemcpy2DAsync(dst + size_t(n1) * es, size_t(ld_dst) * es, ring,
+                                    size_t(ring_len) * es, size_t(n - n1) * es, size_t(n_chans),
+                                    cudaMemcpyDeviceToDevice, s));
+  return PARRM_OK;
 }
 
 }  // extern "C"

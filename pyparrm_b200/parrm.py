@@ -40,6 +40,7 @@ _GRID_LAMBDA = 1.0                       # parrm.py:296
 _N_RESTARTS = 5                          # parrm.py:499
 _HALF_WIDTH_MATCHES = 50                 # parrm.py:792
 _DIRECTIONS = ["both", "past", "future"]  # parrm.py:781
+_DEVICE_DTYPES = ("torch.float64", "torch.float32", "torch.int16", "torch.int32")
 
 _NO_PERIOD_MSG = (
     "The period cannot be estimated from the data. Check that your data "
@@ -69,7 +70,11 @@ class PARRM:
 
     Parameters
     ----------
-    data : numpy.ndarray, shape [channels, times]
+    data : numpy.ndarray, shape [channels, times]; or a CUDA ``torch.Tensor`` (additive)
+        A CUDA tensor (float64 / float32, or int16 / int32 for ``filter_data()`` only) on the
+        engine's GPU is searched and filtered where it lies: nothing crosses PCIe, and
+        ``filter_data()`` / ``_standard_data`` are CUDA tensors.  ``find_period()`` gives
+        bit for bit the period and fit errors of the NumPy array of the same values.
     sampling_freq, artefact_freq : int | float, in Hz
     verbose : bool (default True)
     precision : ``"fp64"`` (default, reference arithmetic) or ``"fp32"`` -- additive,
@@ -111,8 +116,17 @@ class PARRM:
 
     # ------------------------------------------------------------------ inputs
     def _check_init_inputs(self, data, sampling_freq, artefact_freq, verbose) -> None:
-        """Constructor checks (reference parrm.py:112-140)."""
-        if not isinstance(data, np.ndarray):
+        """Constructor checks (reference parrm.py:112-140), plus CUDA-tensor recordings."""
+        if _is_device_tensor(data):
+            if str(data.dtype) not in _DEVICE_DTYPES:
+                raise TypeError(
+                    f"A CUDA tensor `data` must be float64, float32, int16 or int32, not "
+                    f"{data.dtype}.")
+            device = getattr(_engine.get_engine(), "device", None)
+            if device is not None and data.device != device:
+                raise ValueError(
+                    f"`data` is on {data.device}, but this process computes on {device}.")
+        elif not isinstance(data, np.ndarray):
             raise TypeError("`data` must be a NumPy array.")
         if data.ndim != 2:
             raise ValueError("`data` must be a 2D array.")
@@ -154,6 +168,11 @@ class PARRM:
         """
         if self._verbose:
             print("\nFinding the artefact period...")
+        if _sharding.active() and _is_device_tensor(self._data):
+            raise NotImplementedError(
+                "find_period() on a CUDA-tensor recording does not shard: the tensor belongs to "
+                "this rank alone, and the sharded search needs the same recording on every "
+                "rank. Call disable_sharding() first, or pass a NumPy array.")
         self._reset_result_attrs()
         self._check_sort_find_stim_period_inputs(
             search_samples, assumed_periods, outlier_boundary, random_seed, n_jobs
@@ -231,7 +250,11 @@ class PARRM:
         """Reference parrm.py:272-280.  Deferred: the device computes the per-channel scale
         and gathers only the fitted columns (``DeviceEngine.prepare_tiles``); the full
         ``[channels, times - 1]`` array is materialised only if ``_standard_data`` is read."""
-        if not (np.issubdtype(self._data.dtype, np.floating)):
+        if _is_device_tensor(self._data):
+            floating = self._data.is_floating_point()
+        else:
+            floating = np.issubdtype(self._data.dtype, np.floating)
+        if not floating:
             # NumPy refuses the in-place true divide on an integer difference
             raise TypeError(
                 "Cannot standardise non-floating data in place "
@@ -520,7 +543,8 @@ class PARRM:
 
         ``data`` may also be a CUDA ``torch.Tensor`` ``[channels, times]`` (additive): it is
         filtered where it lies and a device tensor comes back -- nothing crosses PCIe (and
-        nothing is sharded: under ``enable_sharding()`` the tensor is this rank's own).
+        nothing is sharded: under ``enable_sharding()`` the tensor is this rank's own).  So is
+        the object's own recording when that is a CUDA tensor and ``data`` is not given.
 
         Under ``pyparrm_b200.enable_sharding()`` every rank filters its channel block (time
         block when channels are fewer than ranks, halos read from the recording); what comes
@@ -535,6 +559,8 @@ class PARRM:
             )
         taps = self._tap_offsets()
         engine = _engine.get_engine()
+        if data is None and _is_device_tensor(self._data):
+            data = self._data  # a CUDA recording is filtered where it lies, as below
         if _is_device_tensor(data):
             # additive overload (SURVEY 8(f).2): a CUDA tensor [channels, times] (float64 or
             # float32) is filtered where it lies and the result stays on the device -- no PCIe
@@ -570,7 +596,7 @@ class PARRM:
         half_width = (self._filter.shape[0] - 1) // 2
         return (np.flatnonzero(self._filter < 0) - half_width).astype(np.int32)
 
-    def filter_stream(self, *, max_chunk=1 << 16, out_dtype=None, graphs=False):
+    def filter_stream(self, *, max_chunk=1 << 16, out_dtype=None, graphs=False, history=0):
         """Filter a recording block by block as it is acquired (additive).
 
         Returns a :class:`pyparrm_b200._stream.FilterStream` holding a snapshot of this
@@ -593,7 +619,25 @@ class PARRM:
         pushes return CUDA tensors in the compute type.  ``graphs=True`` replays NumPy pushes of a
         repeated shape as one CUDA graph (H2D, kernel, D2H); the results are the same bit for
         bit, but on a B200 it measured 8-18 us slower per push than the default separate
-        launches (profiles/r3/stream_latency.txt).  Not available under ``enable_sharding()``."""
+        launches (profiles/r3/stream_latency.txt).  Not available under ``enable_sharding()``.
+
+        ``history``: samples per channel the stream keeps on the device for
+        ``stream.recent(n)``, ``n <= history``, so that the filter can be re-calibrated from the
+        stream's own recent samples and switched in with ``stream.set_filter(cal)``::
+
+            stream = parrm.filter_stream(history=10 * fs)    # keep the last 10 s on the device
+            for block in acquisition:
+                y = stream.push(block)
+                if settings_changed:                        # e.g. a new stimulation frequency
+                    cal = PARRM(stream.recent(10 * fs), fs, new_fa, verbose=False)
+                    cal.find_period()                       # on the GPU, no PCIe
+                    cal.create_filter(filter_half_width=hw, filter_direction="future")
+                    stream.set_filter(cal)                  # outputs not yet returned: new taps
+
+        ``create_filter()`` bounds ``filter_half_width`` by ``(n - 1) // 2`` of the window it was
+        calibrated on, so the window must hold at least ``2 * filter_half_width + 1`` samples.
+        The ring then holds ``max(span, history) + max_chunk`` samples per channel; with
+        ``history=0`` (default) it, the launches and the push times are as without it."""
         if self._filter is None:
             raise ValueError(
                 "The filter has not yet been created. The `create_filter` method must "
@@ -607,7 +651,8 @@ class PARRM:
         from ._stream import FilterStream
 
         return FilterStream(_engine.get_engine(), self._tap_offsets(), self._precision,
-                            max_chunk=max_chunk, out_dtype=out_dtype, graphs=graphs)
+                            max_chunk=max_chunk, out_dtype=out_dtype, graphs=graphs,
+                            history=history)
 
     def filter_sweep(self, parameter_sets, data=None):
         """Filter with many parameter sets at once (additive; SURVEY 8(f).4).
