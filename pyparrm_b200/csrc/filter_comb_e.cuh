@@ -373,6 +373,19 @@ __device__ __forceinline__ int run_block(Rings& r, Walk& w, const Args& a,
         op[s * D] = y;
       } else if (mode != 0) {
         const int64_t t = Tb + c + int64_t(s) * D;
+        if (ES == 4 && mode == 2) {
+          // float32 at a recording edge: the sums are re-added from the rings on every step.
+          // Where the window runs off the end of the recording, n_in falls to 1 while a running
+          // sum still carries the rounding of up to 2B updates of the full window (~n_taps |x|
+          // each) since the block began; divided by n_in that is ~2B n_taps eps32 |x|, above
+          // 1e-4 of the input scale for the cfg4 taps.  Re-added, only the rounding of the
+          // in-range values is left.  (float64 keeps the running sums: 2^-29 times smaller.)
+          r.S0 = ring_sum0(r, s);
+          r.S1 = ring_sum1(r, s);
+          tot = r.S0;
+          if (NK > 1) tot += r.S1;
+          if (NPLUS > 0 || NMINUS > 0 || CENTRE != 0) tot += single;
+        }
         T y = mode == 1 ? fma(tot, neg_inv_n, xc) : edge_value(a.count, a.recip, t, a.n_total, xc, tot);
         if (__builtin_expect(!(fabs(y) <= t_max), 0)) {
           r.S0 = ring_sum0(r, s);

@@ -206,6 +206,39 @@ def test_pattern_first_non_finite_window(case):
     assert np.abs(got - want).max() <= 1e-3  # 1e12 outlier: rounding residue ~1e12 * 2^-52 * steps
 
 
+def test_fp32_specialisations_the_gpu_tests_rely_on():
+    """tests/test_gpu_fp32.py runs the float32 comb kernel on the tap sets of
+    tests/test_gpu_filter.py because float32 gets specialisations that float64 does not
+    (comb_e_shape picks the chunk, the block and the CTAs per SM from the element size).  This
+    asserts that those cases still reach what that file claims for them, with the shape check
+    alone (nothing compiled): if the shape choice changes, it names the coverage that moved."""
+    from tests.test_gpu_filter import SPECIALISED_CASES, _case_taps
+
+    def shape(name, dtype):
+        plan, _ = _native.plan_filter(_case_taps(name), dtype)
+        s = np.zeros(12, dtype=np.int32)
+        status = _native.lib.parrm_filter_specialise_check(plan.ctypes.data, dtype, None,
+                                                           s.ctypes.data, None)
+        assert status == 0, (name, dtype, _native.last_error())
+        m0, u = int(s[2]), int(s[7])
+        return {"plan": tuple(int(v) for v in s[:7]), "m0": m0, "u": u,
+                "b": u * -(-m0 // u), "ctas": int(s[9])}
+
+    f32 = {name: shape(name, _native.F32) for name in SPECIALISED_CASES}
+    f64 = {name: shape(name, _native.F64) for name in SPECIALISED_CASES}
+    # an unrolled block longer than the box (unaligned rows and time shards use this case)
+    assert f32["cfg4 future"]["b"] != f32["cfg4 future"]["m0"], f32["cfg4 future"]
+    assert f32["cfg4 future"]["u"] != f64["cfg4 future"]["u"]
+    # three CTAs per SM, which float64 never gets (time shards, host pipeline, non-finite)
+    assert f32["cfg2"]["ctas"] == 3 and f64["cfg2"]["ctas"] == 2
+    assert all(s["ctas"] <= 2 for s in f64.values())
+    # another plan than float64's: the planner's register bound depends on the element size
+    for name in ("example default", "ecog-like"):
+        assert f32[name]["plan"] != f64[name]["plan"], name
+    # the short one-sided filter: the longest chunk in float32 (unaligned rows use it)
+    assert f32["short future"]["u"] > f64["short future"]["u"]
+
+
 def test_specialisation_threshold_grows_with_the_plan():
     """The job size from which the kernel is compiled for the plan (NVRTC: 0.5 s for the
     BASELINE tap sets, 22 s for 860 taps in runs of 41) scales with the square of the plan's
