@@ -13,6 +13,7 @@
 #include "common.cuh"
 #include "filter_jit.h"
 #include "filter_plan.h"
+#include "gather.cuh"
 
 namespace parrm {
 
@@ -31,21 +32,9 @@ struct FilterArgs {
   int32_t tile;
 };
 
-constexpr int kFilterThreads = 256;
-constexpr int kOutPerThread = 4;
-
-__host__ __device__ inline int round16(int bytes) { return (bytes + 15) & ~15; }
-
-// parrm.py:869: outputs that are not finite become 0 (a NaN/Inf sample zeroes exactly the
-// outputs whose tap window, or own sample, contains it)
-template <typename T>
-__device__ __forceinline__ T finite_or_zero(T y) {
-  return isfinite(y) ? y : T(0);
-}
-
 // ---- shared-memory gather --------------------------------------------------------
 template <typename T>
-__global__ void __launch_bounds__(kFilterThreads)
+__global__ void __launch_bounds__(kGatherThreads)
 filter_gather_smem_kernel(const FilterArgs<T> a) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
@@ -82,81 +71,33 @@ filter_gather_smem_kernel(const FilterArgs<T> a) {
     mbar_expect_tx(bar, uint32_t(n_bulk) * sizeof(T));
     bulk_g2s(s_x + (v_lo - g_lo) + head, xrow + v_lo + head, uint32_t(n_bulk) * sizeof(T), bar);
   }
-  for (int i = tid; i < a.n_taps; i += kFilterThreads) s_taps[i] = a.taps[i];
+  for (int i = tid; i < a.n_taps; i += kGatherThreads) s_taps[i] = a.taps[i];
   // scalar head / tail around the bulk copy, zero fill outside the recording
   if (tid < head) s_x[(v_lo - g_lo) + tid] = xrow[v_lo + tid];
-  for (int i = head + n_bulk + tid; i < n_valid; i += kFilterThreads)
+  for (int i = head + n_bulk + tid; i < n_valid; i += kGatherThreads)
     s_x[(v_lo - g_lo) + i] = xrow[v_lo + i];
-  for (int i = tid; i < int(v_lo - g_lo); i += kFilterThreads) s_x[i] = T(0);
-  for (int i = int(v_hi - g_lo) + tid; i < int(g_hi - g_lo); i += kFilterThreads) s_x[i] = T(0);
+  for (int i = tid; i < int(v_lo - g_lo); i += kGatherThreads) s_x[i] = T(0);
+  for (int i = int(v_hi - g_lo) + tid; i < int(g_hi - g_lo); i += kGatherThreads) s_x[i] = T(0);
   __syncthreads();
   if (n_bulk > 0) mbar_wait(bar, 0);
 
-  const T* s_c = s_x + a.w_hi;  // s_c[i] = sample at tile_t0 + i
   T* orow = a.out + chan * a.ld_out + (tile_t0 - a.t0);
   const bool interior = (g_lo >= 0) && (g_hi <= a.n_total);
-  const int n_taps = a.n_taps;
-
-  if (interior) {
-    const T inv_scale = T(n_taps);
-    for (int i0 = tid; i0 < n_tile; i0 += kFilterThreads * kOutPerThread) {
-      T acc[kOutPerThread];
-#pragma unroll
-      for (int r = 0; r < kOutPerThread; ++r) acc[r] = T(0);
-      // clamp the per-thread outputs of a ragged last pass onto a valid one
-      int idx[kOutPerThread];
-#pragma unroll
-      for (int r = 0; r < kOutPerThread; ++r)
-        idx[r] = min(i0 + r * kFilterThreads, n_tile - 1);
-#pragma unroll 4
-      for (int k = 0; k < n_taps; ++k) {
-        const int w = s_taps[k];
-#pragma unroll
-        for (int r = 0; r < kOutPerThread; ++r) acc[r] += s_c[idx[r] - w];
-      }
-#pragma unroll
-      for (int r = 0; r < kOutPerThread; ++r) {
-        const int i = i0 + r * kFilterThreads;
-        if (i < n_tile) orow[i] = finite_or_zero(s_c[i] - acc[r] / inv_scale);
-      }
-    }
-  } else {
-    for (int i = tid; i < n_tile; i += kFilterThreads) {
-      const int64_t t = tile_t0 + i;
-      T acc = T(0);
-      int n_in = 0;
-      for (int k = 0; k < n_taps; ++k) {
-        const int w = s_taps[k];
-        const int64_t src = t - w;
-        if (src >= 0 && src < a.n_total) {
-          acc += s_c[i - w];
-          ++n_in;
-        }
-      }
-      orow[i] = n_in > 0 ? finite_or_zero(s_c[i] - acc / T(n_in)) : T(0);
-    }
-  }
+  gather_tile<T>(s_x + a.w_hi, s_taps, a.n_taps, n_tile, interior, tile_t0, a.n_total,
+                 [=](int i, T y) { orow[i] = y; });
 }
 
 // ---- global-memory gather (spans or tap lists too large for shared memory) --------
 template <typename T>
-__global__ void __launch_bounds__(kFilterThreads)
+__global__ void __launch_bounds__(kGatherThreads)
 filter_gather_global_kernel(const FilterArgs<T> a) {
   const int64_t chan = blockIdx.y;
   const T* xrow = a.x + chan * a.ld_x - a.x_t0;
   T* orow = a.out + chan * a.ld_out - a.t0;
-  for (int64_t t = a.t0 + int64_t(blockIdx.x) * kFilterThreads + threadIdx.x; t < a.t0 + a.n_out;
-       t += int64_t(gridDim.x) * kFilterThreads) {
-    T acc = T(0);
-    int n_in = 0;
-    for (int k = 0; k < a.n_taps; ++k) {
-      const int64_t src = t - a.taps[k];
-      if (src >= 0 && src < a.n_total) {
-        acc += xrow[src];
-        ++n_in;
-      }
-    }
-    orow[t] = n_in > 0 ? finite_or_zero(xrow[t] - acc / T(n_in)) : T(0);
+  for (int64_t t = a.t0 + int64_t(blockIdx.x) * kGatherThreads + threadIdx.x; t < a.t0 + a.n_out;
+       t += int64_t(gridDim.x) * kGatherThreads) {
+    orow[t] = gather_point<T>(t, a.taps, a.n_taps, a.n_total,
+                              [=](int64_t src) { return xrow[src]; });
   }
 }
 
@@ -165,9 +106,9 @@ filter_gather_global_kernel(const FilterArgs<T> a) {
 // (half-width, period half-width, omit, direction) sets.  blockIdx.z is the set; its taps and
 // tap count are read from device memory (straight from parrm_build_taps_batch, no host round
 // trip); the staged window is sized for the widest set.  Every output counts its in-range
-// taps (the edge form of the kernel above): this path is for small data, not for throughput.
+// taps (the edge form of gather_tile): this path is for small data, not for throughput.
 template <typename T>
-__global__ void __launch_bounds__(kFilterThreads)
+__global__ void __launch_bounds__(kGatherThreads)
 filter_gather_batch_kernel(const T* __restrict__ x, int64_t ld_x, int64_t n_total,
                            const int32_t* __restrict__ taps, int64_t tap_stride,
                            const int32_t* __restrict__ n_taps_of, int32_t w_max, int32_t tile,
@@ -180,30 +121,16 @@ filter_gather_batch_kernel(const T* __restrict__ x, int64_t ld_x, int64_t n_tota
   const int n_tile = int(min64(tile, n_total - t_lo));
   const int n_taps = n_taps_of[set];
   const T* const row = x + chan * ld_x;
-  for (int i = threadIdx.x; i < n_tile + 2 * w_max; i += kFilterThreads) {
+  for (int i = threadIdx.x; i < n_tile + 2 * w_max; i += kGatherThreads) {
     const int64_t g = t_lo - w_max + i;
     s_win[i] = (g >= 0 && g < n_total) ? row[g] : T(0);
   }
-  for (int i = threadIdx.x; i < n_taps; i += kFilterThreads) s_taps[i] = taps[set * tap_stride + i];
+  for (int i = threadIdx.x; i < n_taps; i += kGatherThreads) s_taps[i] = taps[set * tap_stride + i];
   __syncthreads();
   T* const orow = out + set * set_stride + chan * ld_out + t_lo;
-  for (int i = threadIdx.x; i < n_tile; i += kFilterThreads) {
-    const int64_t t = t_lo + i;
-    T acc = T(0);
-    int n_in = 0;
-    for (int k = 0; k < n_taps; ++k) {
-      const int w = s_taps[k];
-      const int64_t src = t - w;
-      if (src >= 0 && src < n_total) {
-        acc += s_win[i + w_max - w];
-        ++n_in;
-      }
-    }
-    orow[i] = n_in > 0 ? finite_or_zero(s_win[i + w_max] - acc / T(n_in)) : T(0);
-  }
+  gather_tile<T>(s_win + w_max, s_taps, n_taps, n_tile, false, t_lo, n_total,
+                 [=](int i, T y) { orow[i] = y; });
 }
-
-constexpr int kSmemBudget = 200 * 1024;
 
 template <typename T>
 int launch_filter(const FilterArgs<T>& args_in, int64_t n_chans, cudaStream_t stream) {
@@ -211,10 +138,10 @@ int launch_filter(const FilterArgs<T>& args_in, int64_t n_chans, cudaStream_t st
   const int64_t span = int64_t(a.w_hi) - a.w_lo;
   const int64_t fixed = 16 + round16(a.n_taps * 4) + 32;
   const int64_t min_window = (1024 + span) * int64_t(sizeof(T));
-  if (fixed + min_window > kSmemBudget) {
-    const int64_t blocks = min64(ceil_div(a.n_out, kFilterThreads), 148 * 32);
+  if (fixed + min_window > kGatherSmemBudget) {
+    const int64_t blocks = min64(ceil_div(a.n_out, kGatherThreads), 148 * 32);
     dim3 grid((unsigned)blocks, (unsigned)n_chans);
-    filter_gather_global_kernel<T><<<grid, kFilterThreads, 0, stream>>>(a);
+    filter_gather_global_kernel<T><<<grid, kGatherThreads, 0, stream>>>(a);
     PARRM_LAUNCH_OK("filter_gather_global_kernel");
     g_last_kernel = "filter_gather_global_kernel";
     return PARRM_OK;
@@ -222,14 +149,14 @@ int launch_filter(const FilterArgs<T>& args_in, int64_t n_chans, cudaStream_t st
   // tile: at least the halo span (<= 2x read amplification from L2), in 1024-output passes
   int64_t tile = ((span + 1023) / 1024) * 1024;
   tile = max64(4096, min64(tile, 8192));
-  while (fixed + (tile + span) * int64_t(sizeof(T)) > kSmemBudget) tile -= 1024;
+  while (fixed + (tile + span) * int64_t(sizeof(T)) > kGatherSmemBudget) tile -= 1024;
   tile = min64(tile, ((a.n_out + 1023) / 1024) * 1024);
   a.tile = int32_t(tile);
   const size_t smem = size_t(fixed + (tile + span + 16 / sizeof(T)) * sizeof(T));
   PARRM_CUDA_OK(cudaFuncSetAttribute(filter_gather_smem_kernel<T>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   dim3 grid((unsigned)ceil_div(a.n_out, tile), (unsigned)n_chans);
-  filter_gather_smem_kernel<T><<<grid, kFilterThreads, smem, stream>>>(a);
+  filter_gather_smem_kernel<T><<<grid, kGatherThreads, smem, stream>>>(a);
   PARRM_LAUNCH_OK("filter_gather_smem_kernel");
   g_last_kernel = "filter_gather_smem_kernel";
   return PARRM_OK;
@@ -377,20 +304,20 @@ int parrm_filter_apply_batch(const void* d_x, int64_t ld_x, int64_t n_samples, i
   PARRM_REQUIRE(max_half_width >= 1 && tap_stride >= 1, "parrm_filter_apply_batch: empty tap rows");
   const int64_t tile = 2048;
   const size_t smem = size_t(tile + 2 * max_half_width) * es + size_t(tap_stride) * 4;
-  PARRM_REQUIRE(smem <= size_t(kSmemBudget),
+  PARRM_REQUIRE(smem <= size_t(kGatherSmemBudget),
                 "parrm_filter_apply_batch: half-width %lld too wide for the batched kernel "
                 "(filter the sets one by one with parrm_filter_apply)", (long long)max_half_width);
   dim3 grid(unsigned(ceil_div(n_samples, tile)), unsigned(n_chans), unsigned(n_sets));
   if (dtype == PARRM_F64) {
     auto kernel = filter_gather_batch_kernel<double>;
     PARRM_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    kernel<<<grid, kFilterThreads, smem, as_stream(stream)>>>(
+    kernel<<<grid, kGatherThreads, smem, as_stream(stream)>>>(
         static_cast<const double*>(d_x), ld_x, n_samples, d_taps, tap_stride, d_n_taps,
         int32_t(max_half_width), int32_t(tile), static_cast<double*>(d_out), ld_out, set_stride);
   } else {
     auto kernel = filter_gather_batch_kernel<float>;
     PARRM_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-    kernel<<<grid, kFilterThreads, smem, as_stream(stream)>>>(
+    kernel<<<grid, kGatherThreads, smem, as_stream(stream)>>>(
         static_cast<const float*>(d_x), ld_x, n_samples, d_taps, tap_stride, d_n_taps,
         int32_t(max_half_width), int32_t(tile), static_cast<float*>(d_out), ld_out, set_stride);
   }

@@ -24,22 +24,17 @@
 // here: no grid-wide barrier is needed.  Work and traffic per push are O(channels x (n + span +
 // pos - out_lo)), independent of how much has been pushed.
 //
-// Arithmetic: the same floating-point operations in the same order as the gather kernels of
-// filter.cu (ascending taps, sequential adds, acc / n_taps in the interior, acc / n_in at the
-// edges, finite_or_zero(x - mean)), so a streamed recording is bit-equal to filter_data with
-// a gather plan on the whole of it.  Widening from the storage type is parrm_convert's
+// Arithmetic: both kernels compute their outputs with the gather body of gather.cuh, the same
+// gather_tile / gather_point that the gather kernels of filter.cu call, so a streamed recording
+// is bit-equal to filter_data with a gather plan on the whole of it by construction.  Only the
+// staging differs (ring + block here).  Widening from the storage type is parrm_convert's
 // static_cast, narrowing to the output type likewise.
 #include <limits.h>
 
 #include "common.cuh"
+#include "gather.cuh"
 
 namespace parrm {
-
-constexpr int kStreamThreads = 256;
-constexpr int kStreamOutPerThread = 4;
-constexpr int kStreamSmemBudget = 200 * 1024;
-
-__host__ __device__ inline int round16s(int bytes) { return (bytes + 15) & ~15; }
 
 template <typename T>
 struct StreamArgs {
@@ -52,11 +47,6 @@ struct StreamArgs {
   int32_t n_taps, w_lo, w_hi, tile;
   int32_t block_type, out_type, close, hdr_words;
 };
-
-template <typename T>
-__device__ __forceinline__ T finite_or_zero_s(T y) {
-  return isfinite(y) ? y : T(0);
-}
 
 template <typename T>
 __device__ __forceinline__ T load_block(const void* b, int type, int64_t i) {
@@ -76,6 +66,16 @@ __device__ __forceinline__ void store_out(void* o, int type, int64_t i, T y) {
     static_cast<float*>(o)[i] = static_cast<float>(y);
 }
 
+// Latency L = max(0, -w_min) of a tap set, and the end of the outputs a push of samples up to
+// `end` makes final: all of them when the stream closes, else those up to end - L.
+__host__ __device__ inline int64_t stream_latency(int32_t w_min) {
+  return w_min < 0 ? -int64_t(w_min) : 0;
+}
+__host__ __device__ inline int64_t stream_out_hi(int64_t end, int64_t out_lo, int64_t lat,
+                                                 int close) {
+  return close ? end : (end - lat > out_lo ? end - lat : out_lo);
+}
+
 // Position, output range and recording end of this push (identical in every CTA).
 struct StreamRange {
   int64_t pos, out_lo, out_hi, n_total;
@@ -84,7 +84,7 @@ struct StreamRange {
 template <typename T>
 __device__ __forceinline__ StreamRange stream_range(const StreamArgs<T>& a) {
   StreamRange r;
-  const int64_t lat = -int64_t(a.w_lo);
+  const int64_t lat = stream_latency(a.w_lo);
   if (a.d_hdr == nullptr) {
     r.pos = a.pos;
     r.out_lo = a.out_lo;
@@ -93,7 +93,7 @@ __device__ __forceinline__ StreamRange stream_range(const StreamArgs<T>& a) {
     r.out_lo = a.hdr_words == 2 ? a.d_hdr[1] : max(int64_t(0), r.pos - lat);
   }
   r.n_total = r.pos + a.n;
-  r.out_hi = a.close ? r.n_total : max(r.out_lo, r.n_total - lat);
+  r.out_hi = stream_out_hi(r.n_total, r.out_lo, lat, a.close);
   return r;
 }
 
@@ -106,7 +106,7 @@ __device__ __forceinline__ void block_to_ring(const StreamArgs<T>& a, const Stre
   if (b0 >= b1) return;
   T* ring = a.ring + chan * a.ring_len;
   const int64_t base = (r.pos + b0) % a.ring_len;  // the slice is shorter than R: one wrap at most
-  for (int64_t i = b0 + threadIdx.x; i < b1; i += kStreamThreads) {
+  for (int64_t i = b0 + threadIdx.x; i < b1; i += kGatherThreads) {
     int64_t j = base + (i - b0);
     if (j >= a.ring_len) j -= a.ring_len;
     ring[j] = load_block<T>(a.block, a.block_type, chan * a.ld_block + i);
@@ -115,11 +115,11 @@ __device__ __forceinline__ void block_to_ring(const StreamArgs<T>& a, const Stre
 
 // ---- shared-memory gather: one output tile + its tap window per CTA ------------------------
 template <typename T>
-__global__ void __launch_bounds__(kStreamThreads)
+__global__ void __launch_bounds__(kGatherThreads)
 stream_gather_smem_kernel(const StreamArgs<T> a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   int32_t* s_taps = reinterpret_cast<int32_t*>(smem_raw);
-  T* s_win = reinterpret_cast<T*>(smem_raw + round16s(a.n_taps * 4));
+  T* s_win = reinterpret_cast<T*>(smem_raw + round16(a.n_taps * 4));
   const int tid = threadIdx.x;
   const int64_t chan = blockIdx.y;
   const StreamRange r = stream_range(a);
@@ -136,8 +136,8 @@ stream_gather_smem_kernel(const StreamArgs<T> a) {
   const T* ring = a.ring + chan * a.ring_len;
   const int64_t ring0 = v_lo % a.ring_len;            // fewer than R samples: one wrap at most
 
-  for (int i = tid; i < a.n_taps; i += kStreamThreads) s_taps[i] = a.taps[i];
-  for (int i = tid; i < int(g_hi - g_lo); i += kStreamThreads) {
+  for (int i = tid; i < a.n_taps; i += kGatherThreads) s_taps[i] = a.taps[i];
+  for (int i = tid; i < int(g_hi - g_lo); i += kGatherThreads) {
     const int64_t g = g_lo + i;
     T v = T(0);
     if (g >= v_lo && g < v_mid) {
@@ -151,57 +151,16 @@ stream_gather_smem_kernel(const StreamArgs<T> a) {
   }
   __syncthreads();
 
-  const T* s_c = s_win + a.w_hi;  // s_c[i] = sample at tile_t0 + i
   const int64_t o0 = chan * a.ld_out + (tile_t0 - r.out_lo);
   const bool interior = (g_lo >= 0) && (g_hi <= r.n_total);
-  const int n_taps = a.n_taps;
-
-  if (interior) {
-    const T inv_scale = T(n_taps);
-    for (int i0 = tid; i0 < n_tile; i0 += kStreamThreads * kStreamOutPerThread) {
-      T acc[kStreamOutPerThread];
-#pragma unroll
-      for (int q = 0; q < kStreamOutPerThread; ++q) acc[q] = T(0);
-      int idx[kStreamOutPerThread];
-#pragma unroll
-      for (int q = 0; q < kStreamOutPerThread; ++q)
-        idx[q] = min(i0 + q * kStreamThreads, n_tile - 1);
-#pragma unroll 4
-      for (int k = 0; k < n_taps; ++k) {
-        const int w = s_taps[k];
-#pragma unroll
-        for (int q = 0; q < kStreamOutPerThread; ++q) acc[q] += s_c[idx[q] - w];
-      }
-#pragma unroll
-      for (int q = 0; q < kStreamOutPerThread; ++q) {
-        const int i = i0 + q * kStreamThreads;
-        if (i < n_tile)
-          store_out(a.out, a.out_type, o0 + i, finite_or_zero_s(s_c[i] - acc[q] / inv_scale));
-      }
-    }
-  } else {
-    for (int i = tid; i < n_tile; i += kStreamThreads) {
-      const int64_t t = tile_t0 + i;
-      T acc = T(0);
-      int n_in = 0;
-      for (int k = 0; k < n_taps; ++k) {
-        const int w = s_taps[k];
-        const int64_t src = t - w;
-        if (src >= 0 && src < r.n_total) {
-          acc += s_c[i - w];
-          ++n_in;
-        }
-      }
-      store_out(a.out, a.out_type, o0 + i,
-                n_in > 0 ? finite_or_zero_s(s_c[i] - acc / T(n_in)) : T(0));
-    }
-  }
+  gather_tile<T>(s_win + a.w_hi, s_taps, a.n_taps, n_tile, interior, tile_t0, r.n_total,
+                 [=](int i, T y) { store_out(a.out, a.out_type, o0 + i, y); });
 }
 
 // ---- global-memory gather: tap windows too wide for shared memory -------------------------
 // The ring of such a stream is read from L2 (384 channels x a 4 k-sample span x 8 B ~ 12 MB).
 template <typename T>
-__global__ void __launch_bounds__(kStreamThreads)
+__global__ void __launch_bounds__(kGatherThreads)
 stream_gather_global_kernel(const StreamArgs<T> a) {
   const int64_t chan = blockIdx.y;
   const StreamRange r = stream_range(a);
@@ -210,19 +169,10 @@ stream_gather_global_kernel(const StreamArgs<T> a) {
   if (t >= r.out_hi) return;
   const T* ring = a.ring + chan * a.ring_len;
   const int64_t blk = chan * a.ld_block - r.pos;  // block element of sample s >= pos: blk + s
-  T acc = T(0);
-  int n_in = 0;
-  for (int k = 0; k < a.n_taps; ++k) {
-    const int64_t src = t - a.taps[k];
-    if (src >= 0 && src < r.n_total) {
-      acc += src >= r.pos ? load_block<T>(a.block, a.block_type, blk + src)
-                          : ring[src % a.ring_len];
-      ++n_in;
-    }
-  }
-  const T x = t >= r.pos ? load_block<T>(a.block, a.block_type, blk + t) : ring[t % a.ring_len];
-  store_out(a.out, a.out_type, chan * a.ld_out + (t - r.out_lo),
-            n_in > 0 ? finite_or_zero_s(x - acc / T(n_in)) : T(0));
+  const T y = gather_point<T>(t, a.taps, a.n_taps, r.n_total, [=](int64_t s) {
+    return s >= r.pos ? load_block<T>(a.block, a.block_type, blk + s) : ring[s % a.ring_len];
+  });
+  store_out(a.out, a.out_type, chan * a.ld_out + (t - r.out_lo), y);
 }
 
 static int64_t stream_span(int32_t w_min, int32_t w_max) {
@@ -233,28 +183,28 @@ template <typename T>
 int launch_stream(StreamArgs<T> a, int64_t n_chans, int64_t n_out_max, cudaStream_t stream) {
   // n_out_max covers both the outputs and the block: CTA x also writes block slice x to the ring
   const int64_t span = int64_t(a.w_hi) - a.w_lo;
-  const int64_t fixed = round16s(a.n_taps * 4);
+  const int64_t fixed = round16(a.n_taps * 4);
   const int64_t es = int64_t(sizeof(T));
-  if (fixed + (kStreamThreads + span) * es > kStreamSmemBudget) {
-    a.tile = kStreamThreads;
+  if (fixed + (kGatherThreads + span) * es > kGatherSmemBudget) {
+    a.tile = kGatherThreads;
     dim3 grid(unsigned(ceil_div(n_out_max, a.tile)), unsigned(n_chans));
-    stream_gather_global_kernel<T><<<grid, kStreamThreads, 0, stream>>>(a);
+    stream_gather_global_kernel<T><<<grid, kGatherThreads, 0, stream>>>(a);
     PARRM_LAUNCH_OK("stream_gather_global_kernel");
     return PARRM_OK;
   }
   // Tiles of 256..4096 outputs: enough CTAs to cover the GPU twice when the push allows it,
   // no more outputs per CTA than the push has, and the window within the shared-memory budget.
   const int64_t want = ceil_div(n_out_max * n_chans, 2 * int64_t(kNumSMs));
-  int64_t tile = ceil_div(max64(want, 1), kStreamThreads) * kStreamThreads;
-  tile = min64(min64(tile, 4096), ceil_div(n_out_max, kStreamThreads) * kStreamThreads);
-  while (tile > kStreamThreads && fixed + (tile + span) * es > kStreamSmemBudget)
-    tile -= kStreamThreads;
+  int64_t tile = ceil_div(max64(want, 1), kGatherThreads) * kGatherThreads;
+  tile = min64(min64(tile, 4096), ceil_div(n_out_max, kGatherThreads) * kGatherThreads);
+  while (tile > kGatherThreads && fixed + (tile + span) * es > kGatherSmemBudget)
+    tile -= kGatherThreads;
   a.tile = int32_t(tile);
   const size_t smem = size_t(fixed + (tile + span) * es);
   PARRM_CUDA_OK(cudaFuncSetAttribute(stream_gather_smem_kernel<T>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
   dim3 grid(unsigned(ceil_div(n_out_max, tile)), unsigned(n_chans));
-  stream_gather_smem_kernel<T><<<grid, kStreamThreads, smem, stream>>>(a);
+  stream_gather_smem_kernel<T><<<grid, kGatherThreads, smem, stream>>>(a);
   PARRM_LAUNCH_OK("stream_gather_smem_kernel");
   return PARRM_OK;
 }
@@ -300,8 +250,7 @@ static int stream_push_impl(const char* fn, void* d_ring, int64_t ring_len, int6
                 (long long)n_chans);
   PARRM_REQUIRE(n_taps >= 1 && w_min <= w_max, "%s: empty or unordered tap list", fn);
   PARRM_REQUIRE(d_ring != nullptr && d_taps != nullptr, "%s: null ring or taps", fn);
-  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
-  const int64_t out_hi = close ? pos + n : (pos + n - lat > out_lo ? pos + n - lat : out_lo);
+  const int64_t out_hi = stream_out_hi(pos + n, out_lo, stream_latency(w_min), close);
   if (n == 0 && out_hi == out_lo) return PARRM_OK;
   PARRM_REQUIRE(n == 0 || (d_block != nullptr && ld_block >= n),
                 "%s: null block or row stride %lld < %lld", fn, (long long)ld_block,
@@ -340,7 +289,7 @@ int parrm_stream_push(void* d_ring, int64_t n_chans, int64_t max_chunk, const in
                 (long long)pos);
   // one tap set for the whole stream: the ring of parrm_stream_ring_bytes and the first output
   // that follows from the position
-  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
+  const int64_t lat = stream_latency(w_min);
   const int64_t out_lo = pos - lat > 0 ? pos - lat : 0;
   const int64_t n_grid = n + (close ? lat : 0);  // grid extent; independent of pos
   return stream_push_impl("parrm_stream_push", d_ring, stream_span(w_min, w_max) + max_chunk,
@@ -373,8 +322,7 @@ int parrm_stream_push_at(void* d_ring, int64_t ring_len, int64_t n_chans, const 
                 "%s: the push reads %lld samples back from pos + n, more than the ring of %lld "
                 "holds (a shorter block, or a longer ring)", fn, (long long)reach,
                 (long long)ring_len);
-  const int64_t lat = w_min < 0 ? -int64_t(w_min) : 0;
-  const int64_t out_hi = close ? pos + n : (pos + n - lat > out_lo ? pos + n - lat : out_lo);
+  const int64_t out_hi = stream_out_hi(pos + n, out_lo, stream_latency(w_min), close);
   const int64_t n_grid = n > out_hi - out_lo ? n : out_hi - out_lo;
   return stream_push_impl(fn, d_ring, ring_len, n_chans, d_taps, n_taps, w_min, w_max, d_block,
                           block_type, ld_block, n, d_out, out_type, ld_out, pos, out_lo, n_grid,
