@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define PARRM_B200_ABI_VERSION 8
+#define PARRM_B200_ABI_VERSION 9
 
 typedef enum {
   PARRM_OK = 0,
@@ -69,6 +69,14 @@ int         parrm_host_is_pinned(const void* h_ptr);
  * copy synchronous with respect to the host, as CUDA defines). */
 int         parrm_copy_h2d_async(void* d_dst, const void* h_src, size_t bytes, void* stream);
 int         parrm_copy_d2h_async(void* h_dst, const void* d_src, size_t bytes, void* stream);
+/* cudaMemcpy2DAsync wrappers: `height` rows of `width` bytes, source rows src_pitch bytes apart,
+ * destination rows dst_pitch bytes apart (both >= width).  They move one time window of a
+ * recording between its place in a larger host array ([C, T] rows, or the [T, ld] rows of a
+ * time-major array) and a dense device buffer, without touching the bytes between the rows. */
+int         parrm_copy_h2d_2d_async(void* d_dst, size_t dst_pitch, const void* h_src,
+                                    size_t src_pitch, size_t width, size_t height, void* stream);
+int         parrm_copy_d2h_2d_async(void* h_dst, size_t dst_pitch, const void* d_src,
+                                    size_t src_pitch, size_t width, size_t height, void* stream);
 /* Page-lock / release a host range in place (cudaHostRegister): a caller that filters or
  * searches the same NumPy array repeatedly registers it once instead of having every call
  * staged through pinned buffers (PARRM holds `data` by reference, parrm.py:124). */
@@ -253,6 +261,17 @@ int parrm_convert_f32_to_f64(const float* d_src, double* d_dst, int64_t n, void*
  * own width and are widened on the device. */
 int parrm_convert(const void* d_src, int src_type, void* d_dst, int dst_type, int64_t n,
                   void* stream);
+/* Transposing convert (csrc/transpose.cu), for time-major recordings -- [times, channels] with
+ * the channels of each sample interleaved, as SpikeGLX / Open Ephys / Intan files and
+ * acquisition APIs deliver them:
+ *     d_dst[c * dst_ld + r] = (dst_type) d_src[r * src_ld + c],  r < rows, c < cols
+ * in one pass through shared-memory tiles.  src_type in {PARRM_F64, PARRM_F32, PARRM_I16,
+ * PARRM_I32}; dst_type is src_type itself, PARRM_F64 or PARRM_F32; each element is converted
+ * with static_cast exactly as parrm_convert does.  Requires src_ld >= cols, dst_ld >= rows and
+ * non-null pointers (else PARRM_ERR_INVALID_ARGUMENT, checked before anything is enqueued); the
+ * source base needs no alignment beyond its element size.  rows or cols 0: nothing to do. */
+int parrm_transpose(const void* d_src, int src_type, int64_t rows, int64_t cols, int64_t src_ld,
+                    void* d_dst, int dst_type, int64_t dst_ld, void* stream);
 
 /* ------------------------------------------------------------------------
  * Streaming filter: filter_data applied block by block as the recording is acquired (an

@@ -27,6 +27,9 @@ _CHUNK_BYTES = int(os.environ.get("PYPARRM_B200_CHUNK_MB", "32")) << 20
 # fewer launches (five kernels per chunk), the copy/compute overlap is the same
 _SEARCH_CHUNK_BYTES = int(os.environ.get("PYPARRM_B200_SEARCH_CHUNK_MB", "128")) << 20
 _PINNED_OUT_LIMIT = int(os.environ.get("PYPARRM_B200_PINNED_OUT_MB", "2048")) << 20
+# a time-major recording is searched from a dense device copy when it takes at most this share
+# of the free device memory (cfg4 in float32: 13.8 GB), else through the host path
+_SEARCH_DEVICE_SHARE = 0.5
 _EVAL_WS_LIMIT = int(os.environ.get("PYPARRM_B200_EVAL_WS_MB", "1024")) << 20
 _N_SLOTS = 3
 _COPY_THREADS = max(1, min(int(os.environ.get("PYPARRM_B200_COPY_THREADS", "8")), (os.cpu_count() or 1)))
@@ -40,6 +43,110 @@ def _threaded_memmove(dst: int, src: int, nbytes: int) -> None:
     """Host-to-host copy between a pageable array and a pinned staging buffer, on the
     library's copy threads (``parrm_host_copy``; the call releases the GIL)."""
     check(lib.parrm_host_copy(_vp(dst), _vp(src), nbytes, _COPY_THREADS), "parrm_host_copy")
+
+
+_copy_pool = None
+_copy_pool_lock = threading.Lock()   # engines of several GPUs may make their first copy at once
+
+
+def _copy_rows(dst: np.ndarray, src: np.ndarray) -> None:
+    """``dst[...] = src`` for 2-D arrays of strided rows (a window of a host array and a dense
+    staging buffer), split by rows over the copy threads (NumPy releases the GIL while it copies)."""
+    global _copy_pool
+    n = dst.shape[0]
+    parts = min(_COPY_THREADS, max(1, dst.nbytes >> 20), n)
+    if parts <= 1:
+        np.copyto(dst, src)
+        return
+    with _copy_pool_lock:
+        if _copy_pool is None:
+            from concurrent.futures import ThreadPoolExecutor
+
+            _copy_pool = ThreadPoolExecutor(_COPY_THREADS, thread_name_prefix="parrm-copy")
+    cuts = [n * i // parts for i in range(parts + 1)]
+    for f in [_copy_pool.submit(np.copyto, dst[a:b], src[a:b]) for a, b in zip(cuts, cuts[1:])]:
+        f.result()
+
+
+# ---------------------------------------------------------------- time-major recordings
+# Raw electrophysiology is stored time-major: int16 [times, channels] with the channels of each
+# sample interleaved (SpikeGLX, Open Ephys, Intan, Blackrock).  Its [channels, times] view
+# (``mm.T``, ``mm[:, a:b].T``) is read as the contiguous rows of the [T, ld] array behind it and
+# transposed on the device (``parrm_transpose``); no host copy of the recording is made.
+
+def time_major_ld(a) -> int | None:
+    """Row pitch ``ld`` in elements when ``a`` is a *time-major* ``[C, T]`` NumPy array -- not
+    C-contiguous, unit channel stride, time stride ``ld * itemsize`` with ``ld >= C``, native
+    byte order -- else None (such arrays keep the C-order path and its host copy)."""
+    if not isinstance(a, np.ndarray) or a.ndim != 2 or a.flags.c_contiguous:
+        return None
+    es = a.dtype.itemsize
+    if not a.dtype.isnative or es == 0 or a.strides[0] != es or a.strides[1] % es:
+        return None
+    ld = a.strides[1] // es
+    return ld if ld >= a.shape[0] else None
+
+
+# A time-major input is read as whole rows of its base, ``ld`` elements per sample for ``C``
+# channels.  Past this ratio the rows carry mostly other channels (one electrode or the sync
+# channel of a 385-channel file: 385x the bytes), and the host copy of the channels asked for is
+# faster.  Measured on a B200 for subsets of a 9 M x 385 int16 file (profiles/r3/time_major.txt):
+# one channel 0.19 s as rows against 0.03 s copied, eight channels 0.16 s against 0.27 s; the
+# copy grows with C, the rows do not, and the two cross near 385 / 64.
+_TIME_MAJOR_MAX_WIDTH = 64
+
+
+def time_major_input_ld(a) -> int | None:
+    """:func:`time_major_ld` of a recording or stream block that is read as the rows of its base:
+    None also when those rows are more than ``_TIME_MAJOR_MAX_WIDTH`` times wider than the
+    channels the view selects (such views keep the host copy)."""
+    ld = time_major_ld(a)
+    return ld if ld is not None and ld <= _TIME_MAJOR_MAX_WIDTH * a.shape[0] else None
+
+
+def window_step(span: int, in_sample_bytes: int, dev_sample_bytes: int) -> int:
+    """Outputs per time window of the windowed filter path, bounded by the bytes a window really
+    moves: about ``_CHUNK_BYTES`` of whichever is larger per sample, the upload
+    (``in_sample_bytes``: ``ld * itemsize`` for a time-major recording) or one device buffer of
+    all channels (``dev_sample_bytes``), and at least ``16 * span``, so the re-sent tap-window
+    halo (``span`` samples) is at most 1/16 of a window (the path is PCIe-bound)."""
+    return max(_CHUNK_BYTES // max(1, in_sample_bytes, dev_sample_bytes), 16 * span, 1)
+
+
+def filter_chunks(n_chans: int, n_samples: int, w_lo: int, w_hi: int, es_in: int, es_out: int,
+                  es_c: int, in_ld: int | None = None, windowed: bool = False) -> list:
+    """``(c0, c1, t0, t1, x0, x1)`` chunks of :meth:`DeviceEngine.filter_host`: channels
+    ``[c0, c1)``, outputs ``[t0, t1)``, inputs ``[x0, x1)``.  ``windowed`` (a time-major
+    recording, ``in_ld`` its row pitch, or an ``out=`` array): time windows of every channel.
+    Otherwise blocks of whole rows, or time windows of one row when a row is long."""
+    span = w_hi - w_lo
+    if windowed:
+        step = window_step(span, (in_ld or n_chans) * es_in, n_chans * max(es_out, es_c))
+        return [(0, n_chans) + w for w in time_windows(n_samples, w_lo, w_hi, step)]
+    row_bytes = n_samples * max(es_in, es_out)
+    if row_bytes <= 2 * _CHUNK_BYTES:
+        rows = max(1, min(n_chans, 65535, _CHUNK_BYTES // row_bytes))
+        return [(c0, min(c0 + rows, n_chans), 0, n_samples, 0, n_samples)
+                for c0 in range(0, n_chans, rows)]
+    step = max(_CHUNK_BYTES // max(es_in, es_out), 4 * span)
+    windows = time_windows(n_samples, w_lo, w_hi, step)
+    return [(c, c + 1) + w for c in range(n_chans) for w in windows]
+
+
+def time_windows(n_samples: int, w_lo: int, w_hi: int, step: int) -> list:
+    """``(t0, t1, x0, x1)`` per window: outputs ``[t0, t1)`` in steps of ``step`` and the inputs
+    ``[x0, x1)`` they read (``y[t]`` reads ``x[t - w]``, ``w_lo <= w <= w_hi``), clipped to the
+    recording."""
+    return [(t0, min(t0 + step, n_samples), max(0, t0 - w_hi),
+             min(n_samples, min(t0 + step, n_samples) - w_lo))
+            for t0 in range(0, n_samples, step)]
+
+
+def time_major_span(ld: int, n_chans: int, x0: int, x1: int, itemsize: int) -> tuple[int, int]:
+    """``(byte offset from the view's first element, bytes)`` of samples ``[x0, x1)`` of every
+    channel of a time-major view: rows ``[x0, x1)`` of its ``[T, ld]`` base, ending at the last
+    channel of row ``x1 - 1`` -- never past the view's last element."""
+    return x0 * ld * itemsize, ((x1 - x0 - 1) * ld + n_chans) * itemsize
 
 
 def pinned_empty(shape, dtype=np.float64) -> np.ndarray:
@@ -123,6 +230,7 @@ class _StreamState:
     stage_in: object = None   # pinned twin of d_in
     d_out: object = None
     stage_out: object = None
+    d_tm: object = None       # a time-major block transposed to [channels, n]
     graphs: dict = field(default_factory=dict)   # push shape -> captured CUDA graph
     seen: set = field(default_factory=set)       # push shapes run once eagerly
     lock: object = field(default_factory=threading.Lock)  # this stream's state, not the engine's
@@ -221,6 +329,9 @@ class DeviceEngine:
         if on_device:
             data, dtype_code = self._device_recording(data)
             elem = data.element_size()
+        elif self._search_on_device(data):
+            data, dtype_code = self._upload_time_major(data)
+            on_device, elem = True, data.element_size()
         else:
             data, dtype_code = self._as_float_array(data, allow_f32=True)
             elem = data.dtype.itemsize
@@ -289,6 +400,59 @@ class DeviceEngine:
             self.s_run.synchronize()
             self._scale = scale
             return self._fp32_tiles(tiles, precision)
+
+    def _search_on_device(self, data: np.ndarray) -> bool:
+        """A float64 / float32 time-major recording is searched from a dense device copy when
+        that copy takes at most ``_SEARCH_DEVICE_SHARE`` of the free device memory; otherwise
+        (and for every other layout) it takes the host path."""
+        if data.dtype not in (np.float64, np.float32) or time_major_input_ld(data) is None:
+            return False
+        free, _ = self.torch.cuda.mem_get_info(self.device)
+        return data.nbytes <= _SEARCH_DEVICE_SHARE * free
+
+    def _upload_time_major(self, data: np.ndarray):
+        """``(dense device [C, T] tensor, dtype code)`` of a float64 / float32 time-major
+        recording, in its own type: time chunks of the rows of its ``[T, ld]`` base go up through
+        the ring and are transposed on the device, with no type change, so the search's device
+        branch reads exactly the values the host path would upload."""
+        t = self.torch
+        ld = time_major_ld(data)
+        n_chans, n_samples = data.shape
+        es = data.dtype.itemsize
+        code = _native.F64 if data.dtype == np.float64 else _native.F32
+        with self._lock, t.cuda.device(self.device):
+            dense = t.empty((n_chans, n_samples), dtype=t.float64 if es == 8 else t.float32,
+                            device=self.device)
+            step = max(1, min(n_samples, _SEARCH_CHUNK_BYTES // (ld * es)))
+            in_bytes = time_major_span(ld, n_chans, 0, step, es)[1]
+            slots = self._slots(in_bytes, 16)
+            pinned = is_pinned(data)
+            stage = None if pinned else self._staging("_stage_in", in_bytes)
+            run = self._stream_ptr(self.s_run)
+            self.s_run.wait_stream(t.cuda.current_stream())
+            for i, x0 in enumerate(range(0, n_samples, step)):
+                x1 = min(x0 + step, n_samples)
+                slot = slots[i % _N_SLOTS]
+                off, nbytes = time_major_span(ld, n_chans, x0, x1, es)
+                src = data.ctypes.data + off
+                if slot["used"]:
+                    slot["ev_run"].synchronize()  # transpose done with d_in (and staging reusable)
+                if not pinned:
+                    _threaded_memmove(stage[i % _N_SLOTS].data_ptr(), src, nbytes)
+                    src = stage[i % _N_SLOTS].data_ptr()
+                check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src), nbytes,
+                                               self._stream_ptr(self.s_in)), "H2D copy")
+                slot["ev_in"].record(self.s_in)
+                self.s_run.wait_event(slot["ev_in"])
+                check(lib.parrm_transpose(_vp(slot["d_in"].data_ptr()), code, x1 - x0, n_chans, ld,
+                                          _vp(dense.data_ptr() + x0 * es), code, n_samples, run),
+                      "parrm_transpose")
+                self._count(1)
+                slot["ev_run"].record(self.s_run)
+                slot["used"] = True
+            t.cuda.current_stream().wait_stream(self.s_run)
+            self.s_run.synchronize()
+        return dense, code
 
     def _fp32_tiles(self, tiles, precision):
         """float32 storage of the tiles in the fp32 mode; channel sums of the rounded values."""
@@ -850,16 +1014,29 @@ class DeviceEngine:
         return self.filter_shard(chunk, taps, x0, t0, t1, n_total).cpu().numpy()
 
     def filter_host(self, data: np.ndarray, taps: np.ndarray, precision: str = "fp64",
-                    strategy: int | None = None, out_dtype=None) -> np.ndarray:
+                    strategy: int | None = None, out_dtype=None, out=None) -> np.ndarray:
         """``filter_data`` body (parrm.py:861-869): NumPy [C, T] in, NumPy [C, T] out (float64
         as the reference returns it, or float32 on request).
 
         Bytes on PCIe: the recording goes up in the caller's dtype (float64, float32, int16 or
         int32) and is widened to the compute type on the device; the result comes back in
-        ``out_dtype``.  ``precision="fp32"`` computes in float32."""
+        ``out_dtype``.  ``precision="fp32"`` computes in float32.
+
+        A time-major recording (:func:`time_major_ld`) goes up as the contiguous rows of its
+        ``[T, ld]`` base, one time window of every channel at a time, and is transposed and
+        widened on the device.  ``out`` (validated by ``PARRM.filter_data``): a float64 / float32
+        ``[C, T]`` array to fill instead of a new one, C-ordered or time-major; the recording
+        then also runs in time windows and a time-major ``out`` gets each window transposed
+        (and narrowed) on the device, then one copy into its rows."""
         t = self.torch
-        data, in_code = self._as_storage_array(data)
+        in_ld = time_major_input_ld(data) if data.dtype.name in self._STORAGE else None
+        if in_ld is None:
+            data, in_code = self._as_storage_array(data)
+        else:
+            in_code = self._STORAGE[data.dtype.name]
         out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
+        if out is not None:
+            out_np = out.dtype
         if out_np not in (np.dtype(np.float64), np.dtype(np.float32)):
             raise TypeError("`out_dtype` must be float64 or float32.")
         comp_code = _native.F32 if precision == "fp32" else _native.F64
@@ -867,92 +1044,134 @@ class DeviceEngine:
         es_in, es_out = data.dtype.itemsize, out_np.itemsize
         es_c = 4 if comp_code == _native.F32 else 8
         n_chans, n_samples = data.shape
-        out = self._output_array((n_chans, n_samples), out_np)
+        windowed = in_ld is not None or out is not None
+        if out is None:
+            out = self._output_array((n_chans, n_samples), out_np)
+        out_ld = time_major_ld(out)
         if n_chans == 0 or n_samples == 0:
             return out
         with self._lock, t.cuda.device(self.device):
             h_plan, d_plan, (w_lo, w_hi) = self._plan(taps, comp_code, strategy)
             opts = self._filter_options(n_chans * n_samples, h_plan=h_plan)
-            span = w_hi - w_lo
-            row_bytes = n_samples * max(es_in, es_out)
-            # chunk list: (c0, c1, t0, t1, x0, x1) -- channels [c0,c1), outputs [t0,t1), inputs [x0,x1)
-            chunks = []
-            if row_bytes <= 2 * _CHUNK_BYTES:
-                rows = max(1, min(n_chans, 65535, _CHUNK_BYTES // row_bytes))
-                for c0 in range(0, n_chans, rows):
-                    chunks.append((c0, min(c0 + rows, n_chans), 0, n_samples, 0, n_samples))
-            else:
-                step = max(_CHUNK_BYTES // max(es_in, es_out), 4 * span)
-                for c in range(n_chans):
-                    for t0 in range(0, n_samples, step):
-                        t1 = min(t0 + step, n_samples)
-                        chunks.append((c, c + 1, t0, t1, max(0, t0 - w_hi), min(n_samples, t1 - w_lo)))
-            in_elems = max((c1 - c0) * (x1 - x0) for c0, c1, _, _, x0, x1 in chunks)
+            chunks = filter_chunks(n_chans, n_samples, w_lo, w_hi, es_in, es_out, es_c, in_ld,
+                                   windowed)
+            in_ptr, out_ptr = data.ctypes.data, out.ctypes.data  # (.ctypes costs microseconds)
+
+            def upload(c0, c1, x0, x1):
+                """(host pointer, pitch, row bytes, rows) of a chunk's input."""
+                if in_ld is not None:
+                    off, nbytes = time_major_span(in_ld, n_chans, x0, x1, es_in)
+                    return in_ptr + off, nbytes, nbytes, 1
+                return (in_ptr + (c0 * n_samples + x0) * es_in, n_samples * es_in,
+                        (x1 - x0) * es_in, c1 - c0)
+
+            def download(c0, c1, t0, t1):
+                """(host pointer, pitch, row bytes, rows) of a chunk's output."""
+                if out_ld is not None:  # rows t0..t1 of the [T, ld] base, channels c0..c1
+                    return (out_ptr + (t0 * out_ld + c0) * es_out, out_ld * es_out,
+                            (c1 - c0) * es_out, t1 - t0)
+                return (out_ptr + (c0 * n_samples + t0) * es_out, n_samples * es_out,
+                        (t1 - t0) * es_out, c1 - c0)
+
+            in_bytes = max(width * height for _, _, width, height in
+                           (upload(c0, c1, x0, x1) for c0, c1, _, _, x0, x1 in chunks))
+            x_elems = max((c1 - c0) * (x1 - x0) for c0, c1, _, _, x0, x1 in chunks)
             out_elems = max((c1 - c0) * (t1 - t0) for c0, c1, t0, t1, _, _ in chunks)
+            tm_in, tm_out = in_ld is not None, out_ld is not None
             widen_in, narrow_out = in_code != comp_code, comp_code != out_code
-            slots = self._slots(in_elems * es_in, out_elems * es_out,
-                                in_elems * es_c if widen_in else 0,
-                                out_elems * es_c if narrow_out else 0)
+            slots = self._slots(in_bytes, out_elems * es_out,
+                                x_elems * es_c if widen_in or tm_in else 0,
+                                out_elems * es_c if narrow_out or tm_out else 0)
             in_pinned, out_pinned = is_pinned(data), is_pinned(out)
-            stage_in = None if in_pinned else self._staging("_stage_in", in_elems * es_in)
+            stage_in = None if in_pinned else self._staging("_stage_in", in_bytes)
             stage_out = None if out_pinned else self._staging("_stage_out", out_elems * es_out)
             s_in, s_run, s_out = (self._stream_ptr(s) for s in (self.s_in, self.s_run, self.s_out))
-            pending = [None] * _N_SLOTS  # (host dst ptr, nbytes) awaiting copy-out of staging
+            pending = [None] * _N_SLOTS  # host destination awaiting copy-out of staging
 
             def drain(k):
                 if pending[k] is not None:
                     slots[k]["ev_out"].synchronize()
-                    dst, nbytes = pending[k]
-                    _threaded_memmove(dst, stage_out[k].data_ptr(), nbytes)
+                    dst, pitch, width, height, (c0, c1, t0, t1) = pending[k]
+                    if pitch == width or height == 1:
+                        _threaded_memmove(dst, stage_out[k].data_ptr(), width * height)
+                    else:
+                        view = out[c0:c1, t0:t1].T if out_ld is not None else out[c0:c1, t0:t1]
+                        staged = stage_out[k][:width * height].numpy().view(out_np)
+                        _copy_rows(view, staged.reshape(view.shape))
                     pending[k] = None
 
             for i, (c0, c1, t0, t1, x0, x1) in enumerate(chunks):
                 k = i % _N_SLOTS
                 slot = slots[k]
                 n_c, n_x, n_o = c1 - c0, x1 - x0, t1 - t0
-                src = data.ctypes.data + (c0 * n_samples + x0) * es_in
-                dst = out.ctypes.data + (c0 * n_samples + t0) * es_out
+                src, pitch, width, height = upload(c0, c1, x0, x1)
                 if slot["used"]:
                     if not in_pinned:
                         slot["ev_in"].synchronize()  # staging buffer free again
                     drain(k)
-                n_in_bytes = n_c * n_x * es_in  # whole rows, or a time window of one row
                 if not in_pinned:
-                    _threaded_memmove(stage_in[k].data_ptr(), src, n_in_bytes)
-                    src = stage_in[k].data_ptr()
+                    if pitch == width or height == 1:
+                        _threaded_memmove(stage_in[k].data_ptr(), src, width * height)
+                    else:  # a time window of a C-order recording's rows
+                        staged = stage_in[k][:width * height].numpy().view(data.dtype)
+                        _copy_rows(staged.reshape(n_c, n_x), data[c0:c1, x0:x1])
+                    src, pitch = stage_in[k].data_ptr(), width
                 if slot["used"]:
                     self.s_in.wait_event(slot["ev_run"])   # kernel finished reading d_in
-                check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src),
-                                               n_in_bytes, s_in), "H2D copy")
+                if pitch == width or height == 1:
+                    check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src),
+                                                   width * height, s_in), "H2D copy")
+                else:
+                    check(lib.parrm_copy_h2d_2d_async(_vp(slot["d_in"].data_ptr()), width,
+                                                      _vp(src), pitch, width, height, s_in),
+                          "H2D copy")
                 slot["ev_in"].record(self.s_in)
                 self.s_run.wait_event(slot["ev_in"])
                 if slot["used"]:
                     self.s_run.wait_event(slot["ev_out"])  # previous result left d_out
                 d_x = slot["d_in"].data_ptr()
-                if widen_in:
+                if tm_in:  # [n_x, ld] rows -> [C, n_x] in the compute type
+                    check(lib.parrm_transpose(_vp(d_x), in_code, n_x, n_c, in_ld,
+                                              _vp(slot["d_x"].data_ptr()), comp_code, n_x, s_run),
+                          "parrm_transpose")
+                    self._count(1)
+                    d_x = slot["d_x"].data_ptr()
+                elif widen_in:
                     check(lib.parrm_convert(_vp(d_x), in_code, _vp(slot["d_x"].data_ptr()),
                                             comp_code, n_c * n_x, s_run), "parrm_convert")
                     self._count(1)
                     d_x = slot["d_x"].data_ptr()
-                d_y = slot["d_y"].data_ptr() if narrow_out else slot["d_out"].data_ptr()
-                self._apply(
-                    opts, _vp(d_x), n_x, x0, n_x, _vp(d_y), n_o, t0, n_o, n_samples,
-                    n_c, _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), comp_code, s_run)
-                self._count(1)
-                if narrow_out:
+                d_y = slot["d_y"].data_ptr() if narrow_out or tm_out else slot["d_out"].data_ptr()
+                for b0 in range(0, n_c, 65535):
+                    n_b = min(65535, n_c - b0)
+                    self._apply(
+                        opts, _vp(d_x + b0 * n_x * es_c), n_x, x0, n_x,
+                        _vp(d_y + b0 * n_o * es_c), n_o, t0, n_o, n_samples, n_b,
+                        _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), comp_code, s_run)
+                    self._count(1)
+                if tm_out:  # [n_c, n_o] -> [n_o, n_c] in the output type
+                    check(lib.parrm_transpose(_vp(d_y), comp_code, n_c, n_o, n_o,
+                                              _vp(slot["d_out"].data_ptr()), out_code, n_c, s_run),
+                          "parrm_transpose")
+                    self._count(1)
+                elif narrow_out:
                     check(lib.parrm_convert(_vp(d_y), comp_code, _vp(slot["d_out"].data_ptr()),
                                             out_code, n_c * n_o, s_run), "parrm_convert")
                     self._count(1)
                 slot["ev_run"].record(self.s_run)
                 self.s_out.wait_event(slot["ev_run"])
-                if out_pinned:
-                    check(lib.parrm_copy_d2h_async(_vp(dst), _vp(slot["d_out"].data_ptr()),
-                                                   n_c * n_o * es_out, s_out), "D2H copy")
+                dst, pitch, width, height = download(c0, c1, t0, t1)
+                d_res = slot["d_out"].data_ptr()
+                if not out_pinned:
+                    check(lib.parrm_copy_d2h_async(_vp(stage_out[k].data_ptr()), _vp(d_res),
+                                                   width * height, s_out), "D2H copy")
+                    pending[k] = (dst, pitch, width, height, (c0, c1, t0, t1))
+                elif pitch == width or height == 1:
+                    check(lib.parrm_copy_d2h_async(_vp(dst), _vp(d_res), width * height, s_out),
+                          "D2H copy")
                 else:
-                    check(lib.parrm_copy_d2h_async(_vp(stage_out[k].data_ptr()),
-                                                   _vp(slot["d_out"].data_ptr()),
-                                                   n_c * n_o * es_out, s_out), "D2H copy")
-                    pending[k] = (dst, n_c * n_o * es_out)
+                    check(lib.parrm_copy_d2h_2d_async(_vp(dst), pitch, _vp(d_res), width, width,
+                                                      height, s_out), "D2H copy")
                 slot["ev_out"].record(self.s_out)
                 slot["used"] = True
             for k in range(_N_SLOTS):
@@ -1062,13 +1281,21 @@ class DeviceEngine:
                 return self._stream_push_device(st, block, pos, close, emitted, output_range)
             if block is None:
                 block = np.zeros((st.n_chans, 0), dtype=np.float64)
-            data, in_code = self._as_storage_array(block)
+            tm_ld = time_major_input_ld(block) if block.dtype.name in self._STORAGE else None
+            if tm_ld is None:
+                data, in_code = self._as_storage_array(block)
+            else:  # its [n, ld] rows go up as they are and are transposed on the device
+                data, in_code = block, self._STORAGE[block.dtype.name]
             n_chans, n = data.shape
             out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
             out_code = _native.F64 if out_np == np.float64 else _native.F32
             lo, hi = output_range(pos, n, st.latency, close, emitted)
             k = hi - lo
             in_bytes, out_bytes = data.nbytes, n_chans * k * out_np.itemsize
+            if tm_ld is not None:
+                in_bytes = time_major_span(tm_ld, n_chans, 0, n, data.dtype.itemsize)[1]
+                if st.d_tm is None or st.d_tm.numel() < data.nbytes:
+                    st.d_tm = self._empty(data.nbytes, t.uint8)
             self._stream_buffers(st, n_chans, in_bytes, out_bytes)
             hdr = self._STREAM_HEADER
             d_in, h_in = st.d_in.data_ptr(), st.stage_in.data_ptr()
@@ -1077,7 +1304,8 @@ class DeviceEngine:
                 _threaded_memmove(h_in + hdr, data.ctypes.data, in_bytes)
             sp = self._stream_ptr(st.stream)
             key = (n_chans, n, in_code, out_code)
-            replayable = graphs and not close and k == n and n > 0
+            # time-major blocks take the eager path (a transpose, then the push kernel)
+            replayable = graphs and tm_ld is None and not close and k == n and n > 0
             if replayable and (key in st.graphs or key in st.seen):
                 st.stage_in[:16].numpy().view(np.int64)[:] = (pos, lo)
                 graph = st.graphs.get(key)
@@ -1090,7 +1318,14 @@ class DeviceEngine:
             else:
                 check(lib.parrm_copy_h2d_async(_vp(d_in + hdr), _vp(h_in + hdr), in_bytes, sp),
                       "H2D copy")
-                self._stream_launch(st, d_in + hdr, in_code, n, n, d_out, out_code, k, pos, lo,
+                d_block = d_in + hdr
+                if tm_ld is not None:  # [n, ld] rows -> [C, n] in the storage type
+                    check(lib.parrm_transpose(_vp(d_block), in_code, n, n_chans, tm_ld,
+                                              _vp(st.d_tm.data_ptr()), in_code, n, sp),
+                          "parrm_transpose")
+                    self._count(1)
+                    d_block = st.d_tm.data_ptr()
+                self._stream_launch(st, d_block, in_code, n, n, d_out, out_code, k, pos, lo,
                                     None, close, sp)
                 self._count(1)
                 check(lib.parrm_copy_d2h_async(_vp(h_out), _vp(d_out), out_bytes, sp), "D2H copy")

@@ -20,7 +20,7 @@ DIR_BOTH, DIR_PAST, DIR_FUTURE = 0, 1, 2
 DIRECTIONS = {"both": DIR_BOTH, "past": DIR_PAST, "future": DIR_FUTURE}
 MAX_BANDWIDTH = 23
 NM_STATE_BYTES = 88
-ABI_VERSION = 8
+ABI_VERSION = 9
 PLAN_AUTO, PLAN_GATHER, PLAN_COMB = 0, 1, 2
 KERNEL_AUTO, KERNEL_GATHER, KERNEL_SPECIALISED = 0, 1, 3
 
@@ -47,6 +47,10 @@ SIGNATURES = {
     "parrm_host_is_pinned": (c_int, [c_void_p]),
     "parrm_copy_h2d_async": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
     "parrm_copy_d2h_async": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
+    "parrm_copy_h2d_2d_async": (
+        c_int, [c_void_p, c_size_t, c_void_p, c_size_t, c_size_t, c_size_t, c_void_p]),
+    "parrm_copy_d2h_2d_async": (
+        c_int, [c_void_p, c_size_t, c_void_p, c_size_t, c_size_t, c_size_t, c_void_p]),
     "parrm_channel_scales_workspace_bytes": (c_size_t, [c_int64, c_int64]),
     "parrm_channel_scales": (
         c_int,
@@ -102,6 +106,8 @@ SIGNATURES = {
     "parrm_host_unregister": (c_int, [c_void_p]),
     "parrm_host_copy": (c_int, [c_void_p, c_void_p, c_size_t, c_int]),
     "parrm_convert": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int64, c_void_p]),
+    "parrm_transpose": (
+        c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_void_p]),
     "parrm_convert_f64_to_f32": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "parrm_convert_f32_to_f64": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
     "parrm_nm_init": (c_int, [c_void_p, c_int32, c_void_p, c_void_p, c_void_p]),

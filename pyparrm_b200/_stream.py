@@ -172,7 +172,12 @@ class FilterStream:
         other real dtypes are converted to float64 -- or a CUDA tensor) and return every output
         that is now final: ``[channels, k]``, NumPy in ``out_dtype`` for NumPy blocks, a CUDA
         tensor in the compute type for CUDA blocks.  Blocks longer than ``max_chunk`` are split
-        here; the channel count is fixed by the first push."""
+        here; the channel count is fixed by the first push.
+
+        A time-major NumPy block -- ``frame.T`` or ``frame[:, :384].T`` of a ``[n, channels]``
+        frame as acquisition APIs deliver it -- crosses into the stream's staging as its
+        contiguous rows and is transposed on the device; the results are the same ``[channels,
+        k]`` arrays, bit for bit.  Such pushes run eagerly also under ``graphs=True``."""
         with self._lock:
             return self._push(block)
 

@@ -13,7 +13,7 @@ FLAGS=(-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17
 # (filter_jit.cu hands it to NVRTC); the same file is also compiled here with its default
 # parameters so that a syntax or resource error shows up at build time.
 { printf 'R"PARRMSRC('; cat "$here/filter_comb_e.cuh"; printf ')PARRMSRC"\n'; } > "$obj/filter_comb_e_src.inc"
-SRCS=(cabi taps filter filter_plan filter_jit standardise period_eval psd neldermead host_copy stream)
+SRCS=(cabi taps filter filter_plan filter_jit standardise period_eval psd neldermead host_copy stream transpose)
 pids=()
 for src in "${SRCS[@]}"; do
   "$NVCC" "${FLAGS[@]}" -c "$here/$src.cu" -o "$obj/$src.o" &

@@ -137,6 +137,28 @@ int parrm_copy_d2h_async(void* h_dst, const void* d_src, size_t bytes, void* str
   return PARRM_OK;
 }
 
+int parrm_copy_h2d_2d_async(void* d_dst, size_t dst_pitch, const void* h_src, size_t src_pitch,
+                            size_t width, size_t height, void* stream) {
+  if (width == 0 || height == 0) return PARRM_OK;
+  PARRM_REQUIRE(d_dst && h_src, "parrm_copy_h2d_2d_async: null pointer");
+  PARRM_REQUIRE(dst_pitch >= width && src_pitch >= width,
+                "parrm_copy_h2d_2d_async: pitch below the row width");
+  PARRM_CUDA_OK(cudaMemcpy2DAsync(d_dst, dst_pitch, h_src, src_pitch, width, height,
+                                  cudaMemcpyHostToDevice, parrm::as_stream(stream)));
+  return PARRM_OK;
+}
+
+int parrm_copy_d2h_2d_async(void* h_dst, size_t dst_pitch, const void* d_src, size_t src_pitch,
+                            size_t width, size_t height, void* stream) {
+  if (width == 0 || height == 0) return PARRM_OK;
+  PARRM_REQUIRE(h_dst && d_src, "parrm_copy_d2h_2d_async: null pointer");
+  PARRM_REQUIRE(dst_pitch >= width && src_pitch >= width,
+                "parrm_copy_d2h_2d_async: pitch below the row width");
+  PARRM_CUDA_OK(cudaMemcpy2DAsync(h_dst, dst_pitch, d_src, src_pitch, width, height,
+                                  cudaMemcpyDeviceToHost, parrm::as_stream(stream)));
+  return PARRM_OK;
+}
+
 int parrm_fp64_fma_burn(int64_t iters, double* d_sink, double* h_flops, void* stream) {
   PARRM_REQUIRE(iters > 0 && d_sink != nullptr, "parrm_fp64_fma_burn: bad arguments");
   const int blocks = parrm::kNumSMs * 8, threads = 256;

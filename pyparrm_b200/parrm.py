@@ -57,6 +57,26 @@ def _require_number(value, name: str) -> None:
         raise TypeError(f"`{name}` must be an int or a float.")
 
 
+def _check_filter_out(out, data: np.ndarray, out_dtype) -> None:
+    """Checks of ``filter_data(out=...)``: a writeable float64 / float32 array of the recording's
+    shape, C-ordered or time-major, sharing no memory with it."""
+    if not isinstance(out, np.ndarray):
+        raise TypeError("`out` must be a NumPy array.")
+    if out.shape != data.shape:
+        raise ValueError(f"`out` must have the shape of `data` {data.shape}, not {out.shape}.")
+    if out.dtype not in (np.dtype(np.float64), np.dtype(np.float32)):
+        raise TypeError(f"`out` must be float64 or float32, not {out.dtype}.")
+    if out_dtype is not None and np.dtype(out_dtype) != out.dtype:
+        raise TypeError(f"`out_dtype` ({np.dtype(out_dtype)}) must match `out.dtype` ({out.dtype}).")
+    if not out.flags.writeable:
+        raise ValueError("`out` must be writeable.")
+    if not out.flags.c_contiguous and _engine.time_major_ld(out) is None:
+        raise ValueError("`out` must be C-contiguous or time-major (the transpose of a "
+                         "[times, channels] array).")
+    if np.may_share_memory(out, data):
+        raise ValueError("`out` must not share memory with `data`.")
+
+
 def _is_device_tensor(obj) -> bool:
     """True for a torch tensor that lives on a CUDA device (without importing torch here)."""
     return (type(obj).__module__.split(".")[0] == "torch" and hasattr(obj, "is_cuda")
@@ -532,7 +552,7 @@ class PARRM:
         filter_[half_width] = 1
         self._filter = filter_
 
-    def filter_data(self, data=None, *, out_dtype=None) -> np.ndarray:
+    def filter_data(self, data=None, *, out_dtype=None, out=None) -> np.ndarray:
         """Apply the PARRM filter and return the result (reference parrm.py:835-875).
 
         Output is float64 ``[channels, times]`` (``out_dtype=numpy.float32``, keyword-only and
@@ -549,7 +569,17 @@ class PARRM:
         Under ``pyparrm_b200.enable_sharding()`` every rank filters its channel block (time
         block when channels are fewer than ranks, halos read from the recording); what comes
         back follows the ``gather`` mode given there, and ``filter_shard`` holds the
-        ``(c0, c1, t0, t1)`` range this rank computed."""
+        ``(c0, c1, t0, t1)`` range this rank computed.
+
+        Time-major recordings -- ``mm.T`` or ``mm[:, a:b].T`` of a ``[times, channels]`` array
+        such as ``np.load("run.npy", mmap_mode="r")``, the layout SpikeGLX / Open Ephys / Intan
+        files hold -- are read as they lie and transposed on the device: no host copy is made.
+
+        ``out`` (keyword-only, additive, NumPy recordings only): a writeable float64 / float32
+        ``[channels, times]`` array to fill and return instead of a new one -- C-ordered, or
+        time-major such as ``np.lib.format.open_memmap(path, "w+", np.float32, (T, C)).T``, which
+        writes the result in the file's own layout.  It must not share memory with ``data``;
+        ``out_dtype``, if given, must be ``out.dtype``."""
         if self._verbose:
             print("Filtering the data...")
         if self._filter is None:
@@ -569,6 +599,9 @@ class PARRM:
                 raise ValueError("`data` must be a 2D array.")
             if out_dtype is not None:
                 raise TypeError("`out_dtype` applies to NumPy results; convert the returned tensor.")
+            if out is not None:
+                raise TypeError("`out` applies to NumPy recordings; a CUDA tensor is filtered "
+                                "into a new device tensor.")
             d_x = data if data.stride(1) == 1 else data.contiguous()
             want = engine.torch.float32 if self._precision == "fp32" else engine.torch.float64
             if d_x.dtype != want:  # float32 / integer recordings are widened, as on the host path
@@ -579,14 +612,21 @@ class PARRM:
                 print("    ... Data filtered\n")
             return self._filtered_data
         data = self._check_sort_filter_data_inputs(data)
+        if out is not None:
+            if _sharding.active():
+                raise NotImplementedError(
+                    "filter_data(out=...) does not shard: call disable_sharding() first, or "
+                    "let filter_data() return its result.")
+            _check_filter_out(out, data, out_dtype)
         if _sharding.active():
-            out, self.filter_shard, _ = _sharding.filter_sharded(
+            result, self.filter_shard, _ = _sharding.filter_sharded(
                 engine, data, taps, self._precision, _sharding.gather_mode(), out_dtype)
-            self._filtered_data = out
+            self._filtered_data = result
         else:
             self.filter_shard = (0, data.shape[0], 0, data.shape[1])
+            extra = {} if out is None else {"out": out}
             self._filtered_data = engine.filter_host(data, taps, self._precision,
-                                                     out_dtype=out_dtype)
+                                                     out_dtype=out_dtype, **extra)
         if self._verbose:
             print("    ... Data filtered\n")
         return self._filtered_data
