@@ -314,6 +314,38 @@ class DeviceEngine:
             setattr(self, which, cur)
         return cur
 
+    def _ring_upload(self, slots, k: int, stage, piece, window=None) -> int:
+        """Put one piece of a host array into ring slot ``k`` on ``s_in`` and make ``s_run``
+        wait for it; returns the slot's device pointer.  ``piece``: ``(host pointer, pitch, row
+        bytes, rows)``.  ``stage``: the pinned staging buffers of a pageable source (None for a
+        pinned one); a strided piece is staged from ``window``, its NumPy view.  A reused
+        slot's staging is refilled once its last copy has left it (the host waits for that
+        copy), and its ``d_in`` once the kernels that read it are done (the copy waits for them
+        on the device).  The caller records the slot's ``ev_run`` after those kernels."""
+        slot = slots[k]
+        src, pitch, width, height = piece
+        if stage is not None:
+            if slot["used"]:
+                slot["ev_in"].synchronize()  # staging buffer free again
+            if pitch == width or height == 1:
+                _threaded_memmove(stage[k].data_ptr(), src, width * height)
+            else:  # a time window of a C-order recording's rows
+                staged = stage[k][:width * height].numpy().view(window.dtype)
+                _copy_rows(staged.reshape(window.shape), window)
+            src, pitch = stage[k].data_ptr(), width
+        if slot["used"]:
+            self.s_in.wait_event(slot["ev_run"])   # kernels finished reading d_in
+        d_in, s_in = slot["d_in"].data_ptr(), self._stream_ptr(self.s_in)
+        if pitch == width or height == 1:
+            check(lib.parrm_copy_h2d_async(_vp(d_in), _vp(src), width * height, s_in), "H2D copy")
+        else:
+            check(lib.parrm_copy_h2d_2d_async(_vp(d_in), width, _vp(src), pitch, width, height,
+                                              s_in), "H2D copy")
+        slot["ev_in"].record(self.s_in)
+        self.s_run.wait_event(slot["ev_in"])
+        slot["used"] = True
+        return d_in
+
     # ------------------------------------------------------------- period search
     def prepare_tiles(
         self, data: np.ndarray, index_sets: list[np.ndarray], outlier_boundary: float,
@@ -354,52 +386,49 @@ class DeviceEngine:
                 )
             rows = max(1, _SEARCH_CHUNK_BYTES // max(1, n_samples * elem))
             rows = min(rows, n_chans, 65535)
-            if on_device:
-                self._device_tiles(data, rows, dtype_code, tiles, outlier_boundary)
+            blocks = [(c0, min(c0 + rows, n_chans)) for c0 in range(0, n_chans, rows)]
+            scale = t.empty(n_chans, dtype=t.float64, device=self.device)
+            ws = self._empty(max(lib.parrm_channel_scales_workspace_bytes(rows, n_samples), 16),
+                             t.uint8)
+            if on_device:  # the host path's channel blocks and row stride, read where they lie
+                sp = self._stream_ptr(t.cuda.current_stream())
+                for c0, c1 in blocks:
+                    block = self._aligned_rows(data, c0, c1)
+                    self._search_block(block.data_ptr(), c0, c1, n_samples, tiles, scale, ws,
+                                       outlier_boundary, dtype_code, sp)
+                t.cuda.current_stream().synchronize()
                 return self._fp32_tiles(tiles, precision)
             in_bytes = rows * n_samples * elem
             slots = self._slots(in_bytes, 16)
-            ws_bytes = lib.parrm_channel_scales_workspace_bytes(rows, n_samples)
-            scale = t.empty(n_chans, dtype=t.float64, device=self.device)
-            ws = self._empty(max(ws_bytes, 16) * _N_SLOTS, t.uint8)
-            pinned = is_pinned(data)
-            stage = None if pinned else self._staging("_stage_in", in_bytes)
+            stage = None if is_pinned(data) else self._staging("_stage_in", in_bytes)
             run = self._stream_ptr(self.s_run)
             self.s_run.wait_stream(t.cuda.current_stream())
-            for i, c0 in enumerate(range(0, n_chans, rows)):
-                c1 = min(c0 + rows, n_chans)
-                slot = slots[i % _N_SLOTS]
+            for i, (c0, c1) in enumerate(blocks):
+                k = i % _N_SLOTS
                 nbytes = (c1 - c0) * n_samples * elem
-                src = data.ctypes.data + c0 * n_samples * elem
-                if slot["used"]:
-                    slot["ev_run"].synchronize()  # kernels done with d_in (and staging reusable)
-                if not pinned:
-                    _threaded_memmove(stage[i % _N_SLOTS].data_ptr(), src, nbytes)
-                    src = stage[i % _N_SLOTS].data_ptr()
-                check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src), nbytes,
-                                               self._stream_ptr(self.s_in)), "H2D copy")
-                slot["ev_in"].record(self.s_in)
-                self.s_run.wait_event(slot["ev_in"])
-                ws_ptr = ws.data_ptr() + (i % _N_SLOTS) * max(ws_bytes, 16)
-                check(lib.parrm_channel_scales(
-                    _vp(slot["d_in"].data_ptr()), c1 - c0, n_samples, n_samples,
-                    _vp(scale.data_ptr() + 8 * c0), _vp(ws_ptr), ws_bytes, dtype_code, run),
-                    "parrm_channel_scales")
-                self._count(2)
-                for tile in tiles:
-                    check(lib.parrm_standardise_gather(
-                        _vp(slot["d_in"].data_ptr()), c1 - c0, n_samples, n_samples,
-                        _vp(tile.indices.data_ptr()), tile.n_indices,
-                        _vp(scale.data_ptr() + 8 * c0), float(outlier_boundary),
-                        _vp(tile.y.data_ptr() + 8 * c0), n_chans,
-                        _vp(tile.sumsq.data_ptr() + 8 * c0), dtype_code, run),
-                        "parrm_standardise_gather")
-                    self._count(2)
-                slot["ev_run"].record(self.s_run)
-                slot["used"] = True
+                d_rows = self._ring_upload(
+                    slots, k, stage, (data.ctypes.data + c0 * n_samples * elem, nbytes, nbytes, 1))
+                self._search_block(d_rows, c0, c1, n_samples, tiles, scale, ws, outlier_boundary,
+                                   dtype_code, run)
+                slots[k]["ev_run"].record(self.s_run)
             self.s_run.synchronize()
-            self._scale = scale
             return self._fp32_tiles(tiles, precision)
+
+    def _search_block(self, d_rows, c0, c1, n_samples, tiles, scale, ws, outlier_boundary, code,
+                      sp) -> None:
+        """Channel scales of the device block ``d_rows`` (channels ``[c0, c1)``, rows
+        ``n_samples`` apart) and the gather of every tile's columns from it, on stream ``sp``."""
+        check(lib.parrm_channel_scales(
+            _vp(d_rows), c1 - c0, n_samples, n_samples, _vp(scale.data_ptr() + 8 * c0),
+            _vp(ws.data_ptr()), ws.numel(), code, sp), "parrm_channel_scales")
+        self._count(2)
+        for tile in tiles:
+            check(lib.parrm_standardise_gather(
+                _vp(d_rows), c1 - c0, n_samples, n_samples, _vp(tile.indices.data_ptr()),
+                tile.n_indices, _vp(scale.data_ptr() + 8 * c0), float(outlier_boundary),
+                _vp(tile.y.data_ptr() + 8 * c0), tile.n_chans, _vp(tile.sumsq.data_ptr() + 8 * c0),
+                code, sp), "parrm_standardise_gather")
+            self._count(2)
 
     def _search_on_device(self, data: np.ndarray) -> bool:
         """A float64 / float32 time-major recording is searched from a dense device copy when
@@ -426,30 +455,20 @@ class DeviceEngine:
             step = max(1, min(n_samples, _SEARCH_CHUNK_BYTES // (ld * es)))
             in_bytes = time_major_span(ld, n_chans, 0, step, es)[1]
             slots = self._slots(in_bytes, 16)
-            pinned = is_pinned(data)
-            stage = None if pinned else self._staging("_stage_in", in_bytes)
+            stage = None if is_pinned(data) else self._staging("_stage_in", in_bytes)
             run = self._stream_ptr(self.s_run)
             self.s_run.wait_stream(t.cuda.current_stream())
             for i, x0 in enumerate(range(0, n_samples, step)):
                 x1 = min(x0 + step, n_samples)
-                slot = slots[i % _N_SLOTS]
+                k = i % _N_SLOTS
                 off, nbytes = time_major_span(ld, n_chans, x0, x1, es)
-                src = data.ctypes.data + off
-                if slot["used"]:
-                    slot["ev_run"].synchronize()  # transpose done with d_in (and staging reusable)
-                if not pinned:
-                    _threaded_memmove(stage[i % _N_SLOTS].data_ptr(), src, nbytes)
-                    src = stage[i % _N_SLOTS].data_ptr()
-                check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src), nbytes,
-                                               self._stream_ptr(self.s_in)), "H2D copy")
-                slot["ev_in"].record(self.s_in)
-                self.s_run.wait_event(slot["ev_in"])
-                check(lib.parrm_transpose(_vp(slot["d_in"].data_ptr()), code, x1 - x0, n_chans, ld,
+                d_rows = self._ring_upload(slots, k, stage,
+                                           (data.ctypes.data + off, nbytes, nbytes, 1))
+                check(lib.parrm_transpose(_vp(d_rows), code, x1 - x0, n_chans, ld,
                                           _vp(dense.data_ptr() + x0 * es), code, n_samples, run),
                       "parrm_transpose")
                 self._count(1)
-                slot["ev_run"].record(self.s_run)
-                slot["used"] = True
+                slots[k]["ev_run"].record(self.s_run)
             t.cuda.current_stream().wait_stream(self.s_run)
             self.s_run.synchronize()
         return dense, code
@@ -472,12 +491,9 @@ class DeviceEngine:
     def _device_recording(self, data):
         """``(rows-contiguous [C, T] tensor, compute code)`` of a float64 / float32 CUDA recording
         on this engine's GPU (a row-strided view is copied to a dense tensor first)."""
-        t = self.torch
         if data.device != self.device:
             raise ValueError(f"the recording is on {data.device}; this engine runs on {self.device}")
-        code = {t.float64: _native.F64, t.float32: _native.F32}.get(data.dtype)
-        if code is None:
-            raise TypeError(f"unsupported data dtype {data.dtype}")
+        code = self._float_code(data)
         if data.dim() != 2:
             raise ValueError("`data` must be a 2D array.")
         if not data.is_contiguous():
@@ -491,35 +507,6 @@ class DeviceEngine:
         so this is what keeps device and host results bit-equal."""
         block = data[c0:c1]
         return block if block.data_ptr() % 16 == 0 else block.clone()
-
-    def _device_tiles(self, data, rows, dtype_code, tiles, outlier_boundary):
-        """The device branch of :meth:`prepare_tiles`: the same channel blocks and row stride as
-        the host path's staging slots, read where the recording lies (no H2D)."""
-        t = self.torch
-        n_chans, n_samples = data.shape
-        sp = self._stream_ptr(t.cuda.current_stream())
-        ws_bytes = lib.parrm_channel_scales_workspace_bytes(rows, n_samples)
-        scale = t.empty(n_chans, dtype=t.float64, device=self.device)
-        ws = self._empty(max(ws_bytes, 16), t.uint8)
-        for c0 in range(0, n_chans, rows):
-            c1 = min(c0 + rows, n_chans)
-            block = self._aligned_rows(data, c0, c1)
-            check(lib.parrm_channel_scales(
-                _vp(block.data_ptr()), c1 - c0, n_samples, n_samples,
-                _vp(scale.data_ptr() + 8 * c0), _vp(ws.data_ptr()), ws_bytes, dtype_code, sp),
-                "parrm_channel_scales")
-            self._count(2)
-            for tile in tiles:
-                check(lib.parrm_standardise_gather(
-                    _vp(block.data_ptr()), c1 - c0, n_samples, n_samples,
-                    _vp(tile.indices.data_ptr()), tile.n_indices,
-                    _vp(scale.data_ptr() + 8 * c0), float(outlier_boundary),
-                    _vp(tile.y.data_ptr() + 8 * c0), n_chans,
-                    _vp(tile.sumsq.data_ptr() + 8 * c0), dtype_code, sp),
-                    "parrm_standardise_gather")
-                self._count(2)
-        t.cuda.current_stream().synchronize()
-        self._scale = scale
 
     def tile_from_standardised(self, z: np.ndarray, indices: np.ndarray) -> SearchTile:
         """Tile from an already standardised ``[channels, times]`` host array (the reference's
@@ -915,6 +902,25 @@ class DeviceEngine:
             data = np.ascontiguousarray(data)
         return data, code
 
+    def _storage_input(self, data: np.ndarray):
+        """``(array, storage code, time-major ld or None)`` of a recording or stream block: a
+        time-major one (:func:`time_major_input_ld`) as it is, to go up as the rows of its base;
+        anything else as :meth:`_as_storage_array` gives it."""
+        ld = time_major_input_ld(data) if data.dtype.name in self._STORAGE else None
+        if ld is None:
+            return (*self._as_storage_array(data), None)
+        return data, self._STORAGE[data.dtype.name], ld
+
+    _TORCH_STORAGE = {"torch.float64": _native.F64, "torch.float32": _native.F32,
+                      "torch.int16": _native.I16, "torch.int32": _native.I32}
+
+    def _float_code(self, tensor) -> int:
+        """Compute type code of a float64 / float32 tensor (TypeError for any other dtype)."""
+        code = self._TORCH_STORAGE.get(str(tensor.dtype))
+        if code not in (_native.F64, _native.F32):
+            raise TypeError(f"unsupported data dtype {tensor.dtype}")
+        return code
+
     # A job of at least this many channel-samples gets the kernel specialised for its plan
     # (built once per plan and device: ~0.5 s for the BASELINE tap sets); smaller one-off jobs
     # keep the pre-built kernels.  The build time grows faster than the unrolled step loop
@@ -958,26 +964,36 @@ class DeviceEngine:
               "parrm_filter_apply_ex")
         self.last_filter_kernel = _native.filter_last_kernel()
 
+    def _filter_rows(self, opts, plan, code, n_chans, d_x, ld_x, x_t0, n_x, d_y, ld_y, t0, n_out,
+                     n_total, sp) -> None:
+        """Filter ``n_chans`` device rows in the compute type ``code``: inputs ``[x_t0, x_t0 +
+        n_x)`` of a recording of ``n_total`` samples at ``d_x`` (rows ``ld_x`` apart) to outputs
+        ``[t0, t0 + n_out)`` at ``d_y`` (rows ``ld_y`` apart), one launch per 65,535 channels."""
+        h_plan, d_plan, _ = plan
+        es = 4 if code == _native.F32 else 8
+        for c0 in range(0, n_chans, 65535):
+            self._apply(
+                opts, _vp(d_x + c0 * ld_x * es), ld_x, x_t0, n_x, _vp(d_y + c0 * ld_y * es), ld_y,
+                t0, n_out, n_total, min(65535, n_chans - c0), _vp(d_plan.data_ptr()),
+                _vp(h_plan.ctypes.data), code, sp)
+            self._count(1)
+
     def filter_device(self, d_x, taps: np.ndarray, d_out=None, stream=None, strategy=None,
                       kernel=None, tuning=None):
         """Filter a device-resident [C, T] tensor (float64 or float32); returns a device tensor."""
         t = self.torch
-        code = {t.float64: _native.F64, t.float32: _native.F32}[d_x.dtype]
+        code = self._float_code(d_x)
         if d_x.dim() != 2 or d_x.stride(1) != 1:
             raise ValueError("device input must be a 2-D row-major tensor")
         n_chans, n_samples = d_x.shape
-        h_plan, d_plan, _ = self._plan(taps, code, strategy)
+        plan = self._plan(taps, code, strategy)
         if d_out is None:
             d_out = t.empty((n_chans, n_samples), dtype=d_x.dtype, device=d_x.device)
         stream = stream or t.cuda.current_stream()
-        opts = self._filter_options(n_chans * n_samples, kernel, tuning, h_plan)
-        for c0 in range(0, n_chans, 65535):
-            c1 = min(c0 + 65535, n_chans)
-            self._apply(
-                opts, _vp(d_x[c0:c1].data_ptr()), d_x.stride(0), 0, n_samples,
-                _vp(d_out[c0:c1].data_ptr()), d_out.stride(0), 0, n_samples, n_samples, c1 - c0,
-                _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), code, self._stream_ptr(stream))
-            self._count(1)
+        opts = self._filter_options(n_chans * n_samples, kernel, tuning, h_plan=plan[0])
+        self._filter_rows(opts, plan, code, n_chans, d_x.data_ptr(), d_x.stride(0), 0, n_samples,
+                          d_out.data_ptr(), d_out.stride(0), 0, n_samples, n_samples,
+                          self._stream_ptr(stream))
         return d_out
 
     def filter_shard(self, chunk: np.ndarray, taps: np.ndarray, x0: int, t0: int, t1: int,
@@ -993,19 +1009,15 @@ class DeviceEngine:
         f32 = precision == "fp32"
         code = _native.F32 if f32 else _native.F64
         with self._lock, t.cuda.device(self.device):
-            h_plan, d_plan, _ = self._plan(taps, code)
+            plan = self._plan(taps, code)
             d_x = t.from_numpy(chunk).to(self.device)
             if f32:
                 d_x = d_x.to(t.float32)
             d_out = t.empty((n_chans, t1 - t0), dtype=d_x.dtype, device=self.device)
-            opts = self._filter_options(n_chans * (t1 - t0), h_plan=h_plan)
-            for c0 in range(0, n_chans, 65535):
-                c1 = min(c0 + 65535, n_chans)
-                self._apply(
-                    opts, _vp(d_x[c0:c1].data_ptr()), n_x, x0, n_x, _vp(d_out[c0:c1].data_ptr()),
-                    t1 - t0, t0, t1 - t0, n_total, c1 - c0, _vp(d_plan.data_ptr()),
-                    _vp(h_plan.ctypes.data), code, self._stream_ptr(t.cuda.current_stream()))
-                self._count(1)
+            opts = self._filter_options(n_chans * (t1 - t0), h_plan=plan[0])
+            self._filter_rows(opts, plan, code, n_chans, d_x.data_ptr(), n_x, x0, n_x,
+                              d_out.data_ptr(), t1 - t0, t0, t1 - t0, n_total,
+                              self._stream_ptr(t.cuda.current_stream()))
             return d_out.to(t.float64)
 
     def filter_host_window(self, chunk: np.ndarray, taps: np.ndarray, x0: int, t0: int, t1: int,
@@ -1029,11 +1041,7 @@ class DeviceEngine:
         then also runs in time windows and a time-major ``out`` gets each window transposed
         (and narrowed) on the device, then one copy into its rows."""
         t = self.torch
-        in_ld = time_major_input_ld(data) if data.dtype.name in self._STORAGE else None
-        if in_ld is None:
-            data, in_code = self._as_storage_array(data)
-        else:
-            in_code = self._STORAGE[data.dtype.name]
+        data, in_code, in_ld = self._storage_input(data)
         out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
         if out is not None:
             out_np = out.dtype
@@ -1051,7 +1059,8 @@ class DeviceEngine:
         if n_chans == 0 or n_samples == 0:
             return out
         with self._lock, t.cuda.device(self.device):
-            h_plan, d_plan, (w_lo, w_hi) = self._plan(taps, comp_code, strategy)
+            plan = self._plan(taps, comp_code, strategy)
+            h_plan, _, (w_lo, w_hi) = plan
             opts = self._filter_options(n_chans * n_samples, h_plan=h_plan)
             chunks = filter_chunks(n_chans, n_samples, w_lo, w_hi, es_in, es_out, es_c, in_ld,
                                    windowed)
@@ -1085,7 +1094,7 @@ class DeviceEngine:
             in_pinned, out_pinned = is_pinned(data), is_pinned(out)
             stage_in = None if in_pinned else self._staging("_stage_in", in_bytes)
             stage_out = None if out_pinned else self._staging("_stage_out", out_elems * es_out)
-            s_in, s_run, s_out = (self._stream_ptr(s) for s in (self.s_in, self.s_run, self.s_out))
+            s_run, s_out = self._stream_ptr(self.s_run), self._stream_ptr(self.s_out)
             pending = [None] * _N_SLOTS  # host destination awaiting copy-out of staging
 
             def drain(k):
@@ -1104,32 +1113,11 @@ class DeviceEngine:
                 k = i % _N_SLOTS
                 slot = slots[k]
                 n_c, n_x, n_o = c1 - c0, x1 - x0, t1 - t0
-                src, pitch, width, height = upload(c0, c1, x0, x1)
                 if slot["used"]:
-                    if not in_pinned:
-                        slot["ev_in"].synchronize()  # staging buffer free again
                     drain(k)
-                if not in_pinned:
-                    if pitch == width or height == 1:
-                        _threaded_memmove(stage_in[k].data_ptr(), src, width * height)
-                    else:  # a time window of a C-order recording's rows
-                        staged = stage_in[k][:width * height].numpy().view(data.dtype)
-                        _copy_rows(staged.reshape(n_c, n_x), data[c0:c1, x0:x1])
-                    src, pitch = stage_in[k].data_ptr(), width
-                if slot["used"]:
-                    self.s_in.wait_event(slot["ev_run"])   # kernel finished reading d_in
-                if pitch == width or height == 1:
-                    check(lib.parrm_copy_h2d_async(_vp(slot["d_in"].data_ptr()), _vp(src),
-                                                   width * height, s_in), "H2D copy")
-                else:
-                    check(lib.parrm_copy_h2d_2d_async(_vp(slot["d_in"].data_ptr()), width,
-                                                      _vp(src), pitch, width, height, s_in),
-                          "H2D copy")
-                slot["ev_in"].record(self.s_in)
-                self.s_run.wait_event(slot["ev_in"])
-                if slot["used"]:
                     self.s_run.wait_event(slot["ev_out"])  # previous result left d_out
-                d_x = slot["d_in"].data_ptr()
+                d_x = self._ring_upload(slots, k, stage_in, upload(c0, c1, x0, x1),
+                                        None if tm_in else data[c0:c1, x0:x1])
                 if tm_in:  # [n_x, ld] rows -> [C, n_x] in the compute type
                     check(lib.parrm_transpose(_vp(d_x), in_code, n_x, n_c, in_ld,
                                               _vp(slot["d_x"].data_ptr()), comp_code, n_x, s_run),
@@ -1142,13 +1130,8 @@ class DeviceEngine:
                     self._count(1)
                     d_x = slot["d_x"].data_ptr()
                 d_y = slot["d_y"].data_ptr() if narrow_out or tm_out else slot["d_out"].data_ptr()
-                for b0 in range(0, n_c, 65535):
-                    n_b = min(65535, n_c - b0)
-                    self._apply(
-                        opts, _vp(d_x + b0 * n_x * es_c), n_x, x0, n_x,
-                        _vp(d_y + b0 * n_o * es_c), n_o, t0, n_o, n_samples, n_b,
-                        _vp(d_plan.data_ptr()), _vp(h_plan.ctypes.data), comp_code, s_run)
-                    self._count(1)
+                self._filter_rows(opts, plan, comp_code, n_c, d_x, n_x, x0, n_x, d_y, n_o, t0, n_o,
+                                  n_samples, s_run)
                 if tm_out:  # [n_c, n_o] -> [n_o, n_c] in the output type
                     check(lib.parrm_transpose(_vp(d_y), comp_code, n_c, n_o, n_o,
                                               _vp(slot["d_out"].data_ptr()), out_code, n_c, s_run),
@@ -1173,7 +1156,6 @@ class DeviceEngine:
                     check(lib.parrm_copy_d2h_2d_async(_vp(dst), pitch, _vp(d_res), width, width,
                                                       height, s_out), "D2H copy")
                 slot["ev_out"].record(self.s_out)
-                slot["used"] = True
             for k in range(_N_SLOTS):
                 drain(k)
             self.s_out.synchronize()
@@ -1281,11 +1263,8 @@ class DeviceEngine:
                 return self._stream_push_device(st, block, pos, close, emitted, output_range)
             if block is None:
                 block = np.zeros((st.n_chans, 0), dtype=np.float64)
-            tm_ld = time_major_input_ld(block) if block.dtype.name in self._STORAGE else None
-            if tm_ld is None:
-                data, in_code = self._as_storage_array(block)
-            else:  # its [n, ld] rows go up as they are and are transposed on the device
-                data, in_code = block, self._STORAGE[block.dtype.name]
+            # a time-major block's [n, ld] rows go up as they are and are transposed on the device
+            data, in_code, tm_ld = self._storage_input(block)
             n_chans, n = data.shape
             out_np = np.dtype(np.float64 if out_dtype is None else out_dtype)
             out_code = _native.F64 if out_np == np.float64 else _native.F32
@@ -1361,9 +1340,6 @@ class DeviceEngine:
             st.graphs.pop(next(iter(st.graphs)))
         st.graphs[key] = graph
         return graph
-
-    _TORCH_STORAGE = {"torch.float64": _native.F64, "torch.float32": _native.F32,
-                      "torch.int16": _native.I16, "torch.int32": _native.I32}
 
     def _stream_push_device(self, st, block, pos, close, emitted, output_range):
         t = self.torch
